@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py - rows/sec of the tabular-DNN train step (BASELINE.json metric) on N B200s.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--config cfg2|cfg1|cfg0] [--impl b200|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--config cfg2|cfg1|cfg0] [--impl b200|reference] [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N --master-addr 127.0.0.1 --master-port P \
            bench.py --gpus N --steps K --warmup W
 
@@ -264,6 +264,8 @@ def main():
     ap.add_argument("--sustained-seconds", type=float, default=3.0)
     ap.add_argument("--e2e-steps", type=int, default=0, help="steps of the host-buffer leg (default: min(steps, 50))")
     ap.add_argument("--also", default="cfg1", help="second config measured on the resident leg only and reported under 'also' ('' = none)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write what the last timed step of --config computed (its loss, the parameters it left) as DIR/*.npy")
     args = ap.parse_args()
     cfg = CONFIGS[args.config]
     rank = int(os.environ.get("RANK", "0"))
@@ -370,9 +372,14 @@ def main():
         t.sync()
         barrier()
         time.sleep(0.3 if full else 0.0)
+        step0 = t.global_step
         ms, wall0, wall1 = timed_run(args.steps, args.warmup)
+        if t.global_step - step0 != args.steps:
+            raise RuntimeError("timed %d steps, --steps asked for %d" % (t.global_step - step0, args.steps))
         clk = sampler.window(wall0, wall1) if (sampler and full) else None
         last_loss = t.last_loss()
+        if full and args.dump_outputs:
+            dump_outputs(args.dump_outputs, t, rank, barrier)
         value = world * B * args.steps / (ms / 1e3)
         res = {"value": value, "ms_per_step": ms / args.steps, "last_loss": last_loss, "clocks": clk,
                "gradient_exchange": exchange, "gpu_launches": t.kernels_per_step(B) * args.steps,
@@ -512,6 +519,22 @@ def main():
         print(json.dumps(out), flush=True)
     if world > 1:
         dist.destroy_process_group()
+
+
+def dump_outputs(out_dir, t, rank, barrier):
+    """What the timed steps hand a caller of sb_trainer_run_resident, taken right after them: the mini-batch loss of the
+    last step (loss.npy, [1]) and the parameters it left (params.npy, the flat layout of sb_trainer_get_params; 10.9 MB
+    at cfg2), both float32.  The inputs (synthetic rows, Xavier init) are seeded, so two builds can be compared file by
+    file; compare with a tolerance, since the order of the step's reductions is not fixed and two runs of one build
+    differ in the last bits (cfg2, 50 + 12 steps: 1.2e-5 max abs on the parameters, on a B200 at 1000 W).  Every rank
+    reads the parameters (a sharded update keeps them on their owner ranks); rank 0 writes."""
+    params = t.get_params()
+    loss = t.loss_history(t.global_step, 1)
+    barrier()
+    if rank == 0:
+        os.makedirs(out_dir, exist_ok=True)
+        np.save(os.path.join(out_dir, "loss.npy"), loss)
+        np.save(os.path.join(out_dir, "params.npy"), params)
 
 
 def ingest_leg(sb, device, hbm_gbs):

@@ -1,5 +1,5 @@
-"""SavedModel / tensor-bundle formats on the CPU: oracle reader vs the reference's own fixture (when present),
-product C++ reader vs oracle reader, product writer -> both readers, golden known answers."""
+"""SavedModel / tensor-bundle formats on the CPU: oracle reader vs the reference's own fixture (shrunk to commit size,
+tests/golden/make_golden.py), product C++ reader vs oracle reader, product writer -> both readers, golden known answers."""
 import json
 import os
 
@@ -9,9 +9,59 @@ import pytest
 from oracle import shifu_oracle as so
 from oracle import tf_formats as tff
 
-FIXTURE = "/root/reference/shifu-tensorflow-eval/src/test/resources/dummydl"
-GOLDEN = os.path.join(os.path.dirname(__file__), "golden", "dummydl_known_answers.json")
-have_fixture = pytest.mark.skipif(not os.path.isdir(FIXTURE), reason="reference fixture only exists in the build container")
+GOLDEN_DIR = os.path.join(os.path.dirname(__file__), "golden")
+GOLDEN = os.path.join(GOLDEN_DIR, "dummydl_known_answers.json")
+HEAD_LAYERS = (0, 1, 2, 20)       # the layers tests/golden/dummydl_head.npz holds whole
+
+
+@pytest.fixture(scope="module")
+def fixture_dir(tmp_path_factory):
+    """The reference's dummydl SavedModel rebuilt from tests/golden: its serving graph and bundle index as TF wrote them,
+    and a data shard of the original length with every stored tensor byte at its original offset.  The kernels of the
+    17 middle layers are a seeded sample there; their other elements read as zeros."""
+    d = tmp_path_factory.mktemp("dummydl")
+    os.makedirs(d / "variables")
+    (d / "saved_model.pb").write_bytes(open(os.path.join(GOLDEN_DIR, "dummydl_serving.pb"), "rb").read())
+    index = open(os.path.join(GOLDEN_DIR, "dummydl_variables.index"), "rb").read()
+    (d / "variables" / "variables.index").write_bytes(index)
+    head = np.load(os.path.join(GOLDEN_DIR, "dummydl_head.npz"))
+    sample = np.load(os.path.join(GOLDEN_DIR, "dummydl_sample.npz"))
+    entries = {}
+    for key, val in tff.read_table(str(d / "variables" / "variables.index")):
+        if key:
+            m = tff.parse_proto(val)
+            entries[key.decode()] = ((tff._fields(m, 4) or [0])[0], (tff._fields(m, 5) or [0])[0])
+    with open(d / "variables" / "variables.data-00000-of-00001", "wb") as f:
+        f.truncate(int(sample["data_bytes"]))
+        for l in range(21):
+            name = "dense_%d/" % (46 + l)
+            if l in HEAD_LAYERS:
+                kernel = head["W%d" % HEAD_LAYERS.index(l)].ravel()
+                spans = [(0, kernel)]
+            else:
+                idx, val = sample["W%d_idx" % l], sample["W%d_val" % l]
+                spans = [(int(i), val[j:j + 1]) for j, i in enumerate(idx)]
+            off, size = entries[name + "kernel"]
+            for i, v in spans:
+                assert 4 * (i + v.size) <= size
+                f.seek(off + 4 * i); f.write(v.astype("<f4").tobytes())
+            off, size = entries[name + "bias"]
+            assert size == 4 * sample["b%d" % l].size
+            f.seek(off); f.write(sample["b%d" % l].astype("<f4").tobytes())
+    return str(d)
+
+
+def _check_against_golden(layers):
+    """every stored value of the fixture read back where it belongs"""
+    head = np.load(os.path.join(GOLDEN_DIR, "dummydl_head.npz"))
+    sample = np.load(os.path.join(GOLDEN_DIR, "dummydl_sample.npz"))
+    for l, (W, b, _act) in enumerate(layers):
+        np.testing.assert_array_equal(b, sample["b%d" % l])
+        if l in HEAD_LAYERS:
+            np.testing.assert_array_equal(W, head["W%d" % HEAD_LAYERS.index(l)])
+        else:
+            np.testing.assert_array_equal(W.ravel()[sample["W%d_idx" % l]], sample["W%d_val" % l])
+    return sample
 
 
 def test_crc32c_known_answers():
@@ -19,38 +69,43 @@ def test_crc32c_known_answers():
     assert tff.crc32c(b"\x00" * 32) == 0x8A9136AA           # RFC 3720 B.4
 
 
-@have_fixture
-def test_oracle_reader_on_reference_fixture_matches_golden():
-    """TensorflowModelTest.java:35-60 loads this model (inputs dense_46_input, output dense_66/Sigmoid)."""
-    layers, names = tff.extract_mlp(FIXTURE, "dense_46_input", "dense_66/Sigmoid")
+def test_oracle_reader_on_reference_fixture_matches_golden(fixture_dir):
+    """TensorflowModelTest.java:35-60 loads this model (inputs dense_46_input, output dense_66/Sigmoid).  The known
+    answers run through the layers the fixture holds whole; the 17 middle layers are bridged by the activations the full
+    model computes there (stored with the fixture)."""
+    layers, names = tff.extract_mlp(fixture_dir, "dense_46_input", "dense_66/Sigmoid")
     assert len(layers) == 21 and layers[0][0].shape == (1522, 100) and layers[-1][0].shape == (100, 1)
     assert [l[2] for l in layers] == [so.ACT_RELU] * 20 + [so.ACT_SIGMOID]
+    assert names == [("dense_%d/kernel" % i, "dense_%d/bias" % i) for i in range(46, 67)]
+    sample = _check_against_golden(layers)
     g = json.load(open(GOLDEN))
+    X = []
     for case in g["cases"]:
         if case["input_fn"] == "const":
-            X = np.full((1, 1522), case["value"], np.float32)
+            X.append(np.full((1, 1522), case["value"], np.float32))
         else:
-            X = np.random.RandomState(case["seed"]).rand(case["rows"], 1522).astype(np.float32)
-        got = tff.mlp_forward(layers, X).ravel()
-        np.testing.assert_allclose(got, np.asarray(case["expected"], np.float32), atol=2e-6)
+            X.append(np.random.RandomState(case["seed"]).rand(case["rows"], 1522).astype(np.float32))
+    X = np.concatenate(X)
+    want = np.concatenate([np.asarray(case["expected"], np.float32) for case in g["cases"]])
+    np.testing.assert_allclose(tff.mlp_forward(layers[:3], X), sample["A3"], atol=2e-6)
+    np.testing.assert_allclose(tff.mlp_forward(layers[20:], sample["A20"]).ravel(), want, atol=2e-6)
 
 
-@have_fixture
-def test_bundle_crcs_of_reference_fixture():
-    b = tff.read_bundle(os.path.join(FIXTURE, "variables", "variables"), verify_crc=False)
+def test_bundle_crcs_of_reference_fixture(fixture_dir):
+    b = tff.read_bundle(os.path.join(fixture_dir, "variables", "variables"), verify_crc=False)
     assert b["dense_46/kernel"].shape == (1522, 100)
     # verify the stored per-tensor crc32c of two tensors (full verify of 27 MB in pure python is slow)
-    entries = dict(tff.read_table(os.path.join(FIXTURE, "variables", "variables.index")))
+    entries = dict(tff.read_table(os.path.join(fixture_dir, "variables", "variables.index")))
     for key in (b"dense_66/bias", b"dense_66/kernel"):
         m = tff.parse_proto(entries[key])
         stored = [v for f, _, v in m if f == 6][0]
         assert tff.crc_mask(tff.crc32c(b[key.decode()].tobytes())) == stored
 
 
-@have_fixture
-def test_cpp_reader_equals_oracle_reader_on_fixture(sb):
-    F, hidden, acts, out_act, flat = sb.capi.savedmodel_read(FIXTURE, "dense_46_input", "dense_66/Sigmoid")
-    layers, _ = tff.extract_mlp(FIXTURE, "dense_46_input", "dense_66/Sigmoid")
+def test_cpp_reader_equals_oracle_reader_on_fixture(sb, fixture_dir):
+    F, hidden, acts, out_act, flat = sb.capi.savedmodel_read(fixture_dir, "dense_46_input", "dense_66/Sigmoid")
+    layers, _ = tff.extract_mlp(fixture_dir, "dense_46_input", "dense_66/Sigmoid")
+    _check_against_golden(layers)
     assert F == 1522 and hidden == [100] * 20 and acts == [so.ACT_RELU] * 20 and out_act == so.ACT_SIGMOID
     ref = np.concatenate([np.concatenate([W.ravel(), b.ravel()]) for W, b, _ in layers])
     np.testing.assert_array_equal(flat, ref)
