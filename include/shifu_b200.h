@@ -165,6 +165,13 @@ int sb_trainer_apply_accumulated_mean(sb_trainer_t* t, int64_t total_pushes);
  * set in RAM and slice mini-batches from it; here the set lives in HBM and each step reads its
  * rows [row_offset, row_offset+rows) from there.  Calling load again replaces the set. */
 int sb_trainer_load_dataset(sb_trainer_t* t, const float* X, const float* y, const float* w, int64_t n_rows);
+/* Wide+deep resident set (after sb_trainer_set_sparse): Xd [n_rows, n_dense] fp32, idx [n_rows, n_cat] int32 (global one-hot
+ * column, -1 = missing), y, w [n_rows]; HOST or DEVICE pointers, like sb_trainer_load_dataset.  Replaces any resident set;
+ * sb_trainer_load_dataset replaces it in turn.  While it is loaded, the resident entry points (step_resident[_async],
+ * run_resident, accumulate_resident, loss_resident, profile_step) run sparse steps.  SB_ERR_STATE before set_sparse,
+ * SB_ERR_INVALID for an index outside [-1, n_onehot) (checked on the device at load; steps do no per-index host work). */
+int sb_trainer_load_dataset_sparse(sb_trainer_t* t, const float* Xd, const int32_t* idx, const float* y, const float* w,
+                                   int64_t n_rows);
 /* (X / y / w of sb_trainer_load_dataset, sb_trainer_eval_loss and sb_trainer_predict may be HOST or DEVICE pointers on the
  * trainer's device: sb_text_parse_device hands the parsed set over without a host round trip.) */
 int sb_trainer_step_resident(sb_trainer_t* t, int64_t row_offset, int32_t rows, float* loss_out);

@@ -107,6 +107,7 @@ PROTOTYPES = {
     "sb_trainer_loss_resident": (C.c_int, [_vp, C.c_int64, C.c_int32, _f32p]),
     "sb_trainer_broadcast_state": (C.c_int, [_vp, C.c_int32]),
     "sb_trainer_load_dataset": (C.c_int, [_vp, _f32p, _f32p, _f32p, C.c_int64]),
+    "sb_trainer_load_dataset_sparse": (C.c_int, [_vp, _f32p, _P(C.c_int32), _f32p, _f32p, C.c_int64]),
     "sb_trainer_step_resident": (C.c_int, [_vp, C.c_int64, C.c_int32, _f32p]),
     "sb_trainer_step_resident_async": (C.c_int, [_vp, C.c_int64, C.c_int32]),
     "sb_trainer_run_resident": (C.c_int, [_vp, C.POINTER(C.c_int64), C.c_int32, C.c_int32]),
@@ -399,6 +400,40 @@ class Trainer:
     def load_dataset(self, X, y, w=None):
         X, y, w, rows = self._xyw(X, y, w)
         check(lib().sb_trainer_load_dataset(self._h, _ptr(X), _ptr(y), _ptr(w), rows))
+        self.dataset_rows = rows
+
+    def load_dataset_sparse(self, Xd, idx, y, w=None):
+        """wide+deep resident set (after set_sparse): Xd [rows, n_dense] and y / w [rows] as numpy or DeviceArray, idx
+        [rows, n_cat] as a numpy integer array or a DeviceArray whose memory holds int32 values.  The resident calls
+        (run_resident, step_resident, accumulate_resident, loss_resident, profile_step) then run sparse steps over it."""
+        if getattr(self, "_sparse", None) is None:      # the library reports the missing set_sparse (SB_ERR_STATE)
+            check(lib().sb_trainer_load_dataset_sparse(self._h, None, None, None, None, 0))
+        n_dense, n_cat = self._sparse
+        if isinstance(Xd, DeviceArray):
+            rows = Xd.shape[0]
+            if len(Xd.shape) != 2 or Xd.shape[1] != n_dense:
+                raise ValueError("Xd must be [rows, %d]" % n_dense)
+        else:
+            Xd = _f32(Xd)
+            rows = Xd.shape[0]
+            if Xd.ndim != 2 or Xd.shape[1] != n_dense:
+                raise ValueError("Xd must be [rows, %d]" % n_dense)
+        if isinstance(idx, DeviceArray):
+            if tuple(idx.shape) != (rows, n_cat):
+                raise ValueError("idx must be [rows, %d]" % n_cat)
+            idx_p = C.cast(idx.ptr, _P(C.c_int32))
+        else:
+            idx = np.ascontiguousarray(idx, dtype=np.int32)
+            if idx.shape != (rows, n_cat):
+                raise ValueError("idx must be [rows, %d]" % n_cat)
+            idx_p = idx.ctypes.data_as(_P(C.c_int32))
+        if not isinstance(y, DeviceArray):
+            y = _f32(y).reshape(-1)
+        if w is not None and not isinstance(w, DeviceArray):
+            w = _f32(w).reshape(-1)
+        if y.size != rows or (w is not None and w.size != rows):
+            raise ValueError("y / w length must equal rows")
+        check(lib().sb_trainer_load_dataset_sparse(self._h, _ptr(Xd), idx_p, _ptr(y), _ptr(w), rows))
         self.dataset_rows = rows
 
     def step_resident(self, row_offset: int, rows: int) -> float:

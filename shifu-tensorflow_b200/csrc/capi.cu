@@ -41,6 +41,10 @@ struct sb_trainer {
   __nv_bfloat16* dsXb = nullptr;                           // bf16 mode: the set in GEMM-operand form [ds_rows, ldF]
   int* dsP = nullptr;                                      // prefix counts of non-zero weights [ds_rows + 1]
   long long ds_rows = 0;
+  // wide+deep set (sb_trainer_load_dataset_sparse): dsX / dsXb hold the dense block (n_dense columns, bf16 pitch ldD),
+  // dsI the index matrix [ds_rows, n_cat]; the resident entry points then run sparse steps
+  int* dsI = nullptr;
+  bool ds_sparse = false;
   std::map<std::pair<int, int>, cudaGraphExec_t> graphs;  // (rows, kind * 2 + from_resident) -> captured step
   std::map<int, int> kernels_per_step;
   // peer-memory exchange (xchg_p2p.cuh): the net's parameter arena [theta | s1 | s2 | shadows | gradient | P2PFlags] is
@@ -278,7 +282,8 @@ static int enqueue_step_body(sb_trainer* t, int rows, int kind, bool resident = 
   // beside each other's persistent GEMMs the "first" order stopped making progress within the exchange timeout)
   const bool order_last = order_last_env || t->peers_share_device;
   static const bool no_defer = getenv("SB_XCHG_NO_DEFER") != nullptr;
-  const bool defer_A = xsched && order_last && resident && n.L >= 3 && !no_defer;
+  // (not for sparse steps: the embedding gather in front of the layer-0 forward GEMM would let it skip a wait it needs)
+  const bool defer_A = xsched && order_last && resident && n.L >= 3 && !no_defer && !sparse;
   if (xsched) {
     n.zero_layer = defer_A ? 1 : 0;
     n.beside_prev_xchg = t->pending_xA;     // slot A's exchange of the previous step is the kernel in front of this step
@@ -461,14 +466,14 @@ static int get_graph(sb_trainer* t, int rows, int kind, bool resident, int pair,
   SB_CUDA(cudaGraphInstantiate(&ge, g, 0));
   cudaGraphDestroy(g);
   t->graphs[key] = ge;
-  if (kind == G_STEP && !sparse && (resident || !t->dsXb)) t->kernels_per_step[rows] = n.launches + 1;  // + set_batch_kernel
+  if (kind == G_STEP && sparse == t->ds_sparse && (resident || !t->dsXb)) t->kernels_per_step[rows] = n.launches + 1;  // + set_batch_kernel
   *out = ge;
   return SB_OK;
 }
 
-// X, y, w are DEVICE pointers here
+// X, y, w (and idx, the index rows of a sparse step) are DEVICE pointers here
 static int run_step(sb_trainer* t, const float* X, const float* y, const float* w, int rows, int kind, long long resident_row0 = -1,
-                    bool sparse = false) {
+                    bool sparse = false, const int* idx = nullptr) {
   Net& n = t->net;
   SB_CHECK(rows > 0 && rows <= n.max_batch, SB_ERR_INVALID, "rows=%d outside (0, max_batch=%d]", rows, n.max_batch);
   SB_CUDA(cudaSetDevice(n.device));
@@ -495,7 +500,7 @@ static int run_step(sb_trainer* t, const float* X, const float* y, const float* 
     if (!t->have_pos) SB_CUDA(cudaEventRecord(t->ev_pos[pair ^ 1], n.stream));
     SB_CUDA(cudaStreamWaitEvent(t->prep, t->ev_pos[pair ^ 1], 0));
     set_batch_kernel<<<1, 1, 0, t->prep>>>(n.desc, nullptr, y, w, lr_t, gscale, t->epoch, static_cast<int>(resident_row0), t->dsP, rows, n.scal,
-                                           kind == G_STEP ? t->hist_slot(t->global_step) : nullptr);
+                                           kind == G_STEP ? t->hist_slot(t->global_step) : nullptr, idx);
     SB_CUDA(cudaGetLastError());
     SB_CUDA(cudaEventRecord(t->ev_prep[pair], t->prep));
     SB_CUDA(cudaEventRecord(t->ev_pos[pair], n.stream));
@@ -506,10 +511,10 @@ static int run_step(sb_trainer* t, const float* X, const float* y, const float* 
     t->have_pos = false;
     if (resident)
       set_batch_kernel<<<1, 1, 0, n.stream>>>(n.desc, nullptr, y, w, lr_t, gscale, t->epoch, static_cast<int>(resident_row0), t->dsP, rows, n.scal,
-                                               kind == G_STEP ? t->hist_slot(t->global_step) : nullptr);
+                                               kind == G_STEP ? t->hist_slot(t->global_step) : nullptr, idx);
     else
       set_batch_kernel<<<1, 1, 0, n.stream>>>(n.desc, X, y, w ? w : n.ones, lr_t, gscale, t->epoch, 0, nullptr, 0, nullptr,
-                                               kind == G_STEP ? t->hist_slot(t->global_step) : nullptr);
+                                               kind == G_STEP ? t->hist_slot(t->global_step) : nullptr, idx);
   }
   SB_CUDA(cudaGetLastError());
   if (no_graph) SB_TRY(enqueue_step_body(t, rows, kind, resident, sparse));
@@ -887,6 +892,7 @@ int sb_trainer_destroy(sb_trainer_t* t) {
   if (t->dsX) cudaFree(t->dsX);
   if (t->dsXb) cudaFree(t->dsXb);
   if (t->dsP) cudaFree(t->dsP);
+  if (t->dsI) cudaFree(t->dsI);
   if (t->dsY) cudaFree(t->dsY);
   if (t->dsW) cudaFree(t->dsW);
   if (t->h_scal) cudaFreeHost(t->h_scal);
@@ -971,6 +977,9 @@ int sb_trainer_step(sb_trainer_t* t, const float* X, const float* y, const float
 // ---- wide+deep (BASELINE config 4): hidden layer 0 = [dense | one-hot]; the step feeds (dense block, index matrix) ----
 int sb_trainer_set_sparse(sb_trainer_t* t, int32_t n_dense, int32_t n_onehot, int32_t n_cat) {
   SB_CHECK(t, SB_ERR_INVALID, "null trainer");
+  const Net& n = t->net;
+  SB_CHECK(!t->ds_sparse || (n_dense == n.n_dense && n_onehot == n.n_onehot && n_cat == n.n_cat), SB_ERR_STATE,
+           "a wide+deep resident set of another shape is loaded; load a set of the new shape after this call instead");
   return t->net.set_sparse(n_dense, n_onehot, n_cat);
 }
 
@@ -992,7 +1001,7 @@ int sb_trainer_step_sparse(sb_trainer_t* t, const float* Xd, const int32_t* idx,
                            float* loss_out) {
   SB_CHECK(t && y, SB_ERR_INVALID, "null argument");
   SB_TRY(stage_sparse_batch(t->net, Xd, idx, y, w, rows));
-  SB_TRY(run_step(t, t->net.stX, t->net.stY, w ? t->net.stW : nullptr, rows, G_STEP, -1, true));
+  SB_TRY(run_step(t, t->net.stX, t->net.stY, w ? t->net.stW : nullptr, rows, G_STEP, -1, true, t->net.idx));
   return finish_loss(t, loss_out);
 }
 
@@ -1005,7 +1014,8 @@ static int forward_chunks_sparse(Net& n, const float* Xd, const int32_t* idx, co
   for (int64_t r0 = 0; r0 < rows; r0 += n.max_batch) {
     const int c = static_cast<int>(rows - r0 < n.max_batch ? rows - r0 : n.max_batch);
     SB_TRY(stage_sparse_batch(n, Xd + r0 * n.n_dense, idx + r0 * n.n_cat, do_loss ? y + r0 : nullptr, (do_loss && w) ? w + r0 : nullptr, c));
-    set_batch_kernel<<<1, 1, 0, n.stream>>>(n.desc, n.stX, n.stY, (do_loss && w) ? n.stW : n.ones, 0.f, 1.f);
+    set_batch_kernel<<<1, 1, 0, n.stream>>>(n.desc, n.stX, n.stY, (do_loss && w) ? n.stW : n.ones, 0.f, 1.f, 0, 0, nullptr, 0, nullptr,
+                                             nullptr, n.idx);
     n.sparse_step = true;
     SB_TRY(n.enqueue_load(c));
     SB_TRY(n.enqueue_hidden_forward(c));
@@ -1115,22 +1125,51 @@ static int apply_accumulated_impl(sb_trainer_t* t, int64_t total_pushes) {
   return SB_OK;
 }
 
-int sb_trainer_load_dataset(sb_trainer_t* t, const float* X, const float* y, const float* w, int64_t n_rows) {
+// The resident set: X [n_rows, cols] fp32, cols = F, or (wide+deep, idx != nullptr) the dense block of n_dense columns beside
+// the index matrix idx [n_rows, n_cat].  Any of the pointers may be HOST or DEVICE memory.
+static int load_resident_set(sb_trainer* t, const float* X, const int32_t* idx, const float* y, const float* w, int64_t n_rows) {
   SB_CHECK(t && X && y, SB_ERR_INVALID, "null argument");
   SB_CHECK(n_rows > 0 && n_rows < (1ll << 31), SB_ERR_INVALID, "n_rows must be in (0, 2^31)");
   Net& n = t->net;
+  const bool sparse = idx != nullptr;
+  const int cols = sparse ? n.n_dense : n.F, ld = sparse ? n.ldD : n.ldF;
   SB_CUDA(cudaSetDevice(n.device));
   SB_CUDA(cudaStreamSynchronize(n.stream));
-  for (auto& kv : t->graphs) cudaGraphExecDestroy(kv.second);   // captured steps carry tensor maps of the old set
-  t->graphs.clear();
-  for (auto& kv : t->run_graphs) cudaGraphExecDestroy(kv.second);
-  t->run_graphs.clear();
+  int* dsI = nullptr;
+  if (sparse) {
+    // copied and range-checked on the device (host and device input alike) before the old set is dropped, so a rejected
+    // set leaves the trainer as it was; steps then do no per-index host work
+    const long long ni = n_rows * static_cast<long long>(n.n_cat);
+    SB_CUDA(cudaMalloc(&dsI, sizeof(int) * ni));
+    int* range = nullptr;
+    int h[2] = {0x7fffffff, -0x7fffffff - 1};
+    cudaError_t e = cudaMalloc(&range, sizeof(h));
+    if (e == cudaSuccess) e = cudaMemcpyAsync(dsI, idx, sizeof(int) * ni, cudaMemcpyDefault, n.stream);
+    if (e == cudaSuccess) e = cudaMemcpyAsync(range, h, sizeof(h), cudaMemcpyHostToDevice, n.stream);
+    if (e == cudaSuccess) {
+      const long long blocks = std::min<long long>((ni + 255) / 256, static_cast<long long>(n.num_sms) * 8);
+      int_range_kernel<<<static_cast<unsigned>(blocks), 256, 0, n.stream>>>(dsI, ni, range);
+      e = cudaGetLastError();
+    }
+    if (e == cudaSuccess) e = cudaMemcpyAsync(h, range, sizeof(h), cudaMemcpyDeviceToHost, n.stream);
+    if (e == cudaSuccess) e = cudaStreamSynchronize(n.stream);
+    if (range) cudaFree(range);
+    if (e != cudaSuccess || h[0] < -1 || h[1] >= n.n_onehot) {
+      cudaFree(dsI);
+      SB_CHECK(e == cudaSuccess, SB_ERR_CUDA, "index matrix copy / range check failed: %s", cudaGetErrorString(e));
+      return set_error(SB_ERR_INVALID, "idx holds values in [%d, %d], outside [-1, n_onehot=%d)", h[0], h[1], n.n_onehot);
+    }
+  }
+  drop_step_graphs(t);   // captured steps carry tensor maps of the old set
   if (t->dsX) cudaFree(t->dsX);
   if (t->dsXb) cudaFree(t->dsXb);
   if (t->dsY) cudaFree(t->dsY);
   if (t->dsW) cudaFree(t->dsW);
   if (t->dsP) cudaFree(t->dsP);
+  if (t->dsI) cudaFree(t->dsI);
   t->dsX = t->dsY = t->dsW = nullptr; t->dsXb = nullptr; t->dsP = nullptr; t->ds_rows = 0;
+  t->dsI = dsI;
+  t->ds_sparse = sparse;
   SB_CUDA(cudaMalloc(&t->dsY, sizeof(float) * n_rows));
   SB_CUDA(cudaMalloc(&t->dsW, sizeof(float) * n_rows));
   SB_CUDA(cudaMemcpyAsync(t->dsY, y, sizeof(float) * n_rows, cudaMemcpyDefault, n.stream));
@@ -1141,22 +1180,22 @@ int sb_trainer_load_dataset(sb_trainer_t* t, const float* X, const float* y, con
     SB_CUDA(cudaGetLastError());
   }
   if (n.tc()) {
-    // keep the set in HBM in the form the layer-0 GEMMs consume (bf16, row pitch ldF; split modes: nparts such arrays):
+    // keep the set in HBM in the form the layer-0 GEMMs consume (bf16, row pitch ld; split modes: nparts such arrays):
     // converted once here, read by TMA every step.  Converted through a bounded fp32 window so a 100+ GB set never needs
     // a second full copy.
-    const size_t part_elems = static_cast<size_t>(n_rows) * n.ldF;
+    const size_t part_elems = static_cast<size_t>(n_rows) * ld;
     SB_CUDA(cudaMalloc(&t->dsXb, sizeof(__nv_bfloat16) * part_elems * n.nparts));
     SB_CUDA(cudaMemsetAsync(t->dsXb, 0, sizeof(__nv_bfloat16) * part_elems * n.nparts, n.stream));
     n.resident_ps = static_cast<long long>(part_elems);
     const int64_t win = 32768;
     float* tmp = nullptr;
-    SB_CUDA(cudaMalloc(&tmp, sizeof(float) * static_cast<size_t>(win < n_rows ? win : n_rows) * n.F));
+    SB_CUDA(cudaMalloc(&tmp, sizeof(float) * static_cast<size_t>(win < n_rows ? win : n_rows) * cols));
     for (int64_t r0 = 0; r0 < n_rows; r0 += win) {
       const int64_t c = n_rows - r0 < win ? n_rows - r0 : win;
-      SB_CUDA(cudaMemcpyAsync(tmp, X + r0 * n.F, sizeof(float) * c * n.F, cudaMemcpyDefault, n.stream));
-      cast_bf16_kernel<<<static_cast<unsigned>((c * n.F + 255) / 256), 256, 0, n.stream>>>(tmp, static_cast<int>(c), n.F,
-                                                                                           t->dsXb + r0 * n.ldF, n.ldF, n.nparts,
-                                                                                           n.resident_ps);
+      SB_CUDA(cudaMemcpyAsync(tmp, X + r0 * cols, sizeof(float) * c * cols, cudaMemcpyDefault, n.stream));
+      cast_bf16_kernel<<<static_cast<unsigned>((c * cols + 255) / 256), 256, 0, n.stream>>>(tmp, static_cast<int>(c), cols,
+                                                                                            t->dsXb + r0 * ld, ld, n.nparts,
+                                                                                            n.resident_ps);
       SB_CUDA(cudaGetLastError());
       SB_CUDA(cudaStreamSynchronize(n.stream));   // X may be pageable: the window is reused
     }
@@ -1177,13 +1216,31 @@ int sb_trainer_load_dataset(sb_trainer_t* t, const float* X, const float* y, con
     n.resident_Xb = t->dsXb;
     n.resident_rows = n_rows;
   } else {
-    SB_CUDA(cudaMalloc(&t->dsX, sizeof(float) * n_rows * n.F));
-    SB_CUDA(cudaMemcpyAsync(t->dsX, X, sizeof(float) * n_rows * n.F, cudaMemcpyDefault, n.stream));
+    SB_CUDA(cudaMalloc(&t->dsX, sizeof(float) * n_rows * cols));
+    SB_CUDA(cudaMemcpyAsync(t->dsX, X, sizeof(float) * n_rows * cols, cudaMemcpyDefault, n.stream));
   }
   SB_CUDA(cudaStreamSynchronize(n.stream));
   t->ds_rows = n_rows;
   return SB_OK;
 }
+
+int sb_trainer_load_dataset(sb_trainer_t* t, const float* X, const float* y, const float* w, int64_t n_rows) {
+  return load_resident_set(t, X, nullptr, y, w, n_rows);
+}
+
+int sb_trainer_load_dataset_sparse(sb_trainer_t* t, const float* Xd, const int32_t* idx, const float* y, const float* w,
+                                   int64_t n_rows) {
+  SB_CHECK(t, SB_ERR_INVALID, "null trainer");
+  SB_CHECK(t->net.n_cat > 0, SB_ERR_STATE, "sb_trainer_set_sparse has not been called");
+  SB_CHECK(idx, SB_ERR_INVALID, "idx must not be null");
+  return load_resident_set(t, Xd, idx, y, w, n_rows);
+}
+
+// fp32 rows / index rows of the resident set from `row` on (nullptr where the set has none)
+static const float* ds_x(const sb_trainer* t, long long row) {
+  return t->dsX ? t->dsX + row * (t->ds_sparse ? t->net.n_dense : t->net.F) : nullptr;
+}
+static const int* ds_idx(const sb_trainer* t, long long row) { return t->dsI ? t->dsI + row * t->net.n_cat : nullptr; }
 
 static int resident_step(sb_trainer_t* t, int64_t row_offset, int32_t rows, int kind) {
   SB_CHECK(t, SB_ERR_INVALID, "null trainer");
@@ -1191,8 +1248,8 @@ static int resident_step(sb_trainer_t* t, int64_t row_offset, int32_t rows, int 
   SB_CHECK(row_offset >= 0 && rows > 0 && row_offset + rows <= t->ds_rows, SB_ERR_INVALID,
            "rows [%lld, %lld) outside the resident set of %lld rows", (long long)row_offset, (long long)(row_offset + rows),
            (long long)t->ds_rows);
-  return run_step(t, t->dsX ? t->dsX + row_offset * t->net.F : nullptr, t->dsY + row_offset, t->dsW + row_offset, rows, kind,
-                  row_offset);
+  return run_step(t, ds_x(t, row_offset), t->dsY + row_offset, t->dsW + row_offset, rows, kind, row_offset, t->ds_sparse,
+                  ds_idx(t, row_offset));
 }
 
 // RUN_S consecutive steps as ONE graph over descriptor set `set`
@@ -1212,7 +1269,7 @@ static int get_run_graph(sb_trainer* t, int rows, int set, cudaGraphExec_t* out)
     // (SB_STEP_TRACE: an interior step is the one traced - with the peer exchange, the last step of a graph joins the
     // exchange of slot A at its end instead of hiding it behind the next step's layer-0 forward)
     n.trace_on = (k == 1);
-    s = enqueue_step_body(t, rows, G_STEP, true, false, k == sb_trainer::RUN_S - 1);
+    s = enqueue_step_body(t, rows, G_STEP, true, t->ds_sparse, k == sb_trainer::RUN_S - 1);
   }
   n.trace_on = true;
   t->pending_xA = false;
@@ -1268,7 +1325,7 @@ int sb_trainer_run_resident(sb_trainer_t* t, const int64_t* row_offsets, int32_t
         ++t->epoch;
         set_batch_kernel<<<1, 1, 0, t->prep>>>(t->run_descs[set][k], nullptr, t->dsY + off, t->dsW + off,
                                                lr_for_step(t, t->global_step), gscale, t->epoch, static_cast<int>(off), t->dsP,
-                                               rows, t->run_scals[set][k], t->hist_slot(t->global_step));
+                                               rows, t->run_scals[set][k], t->hist_slot(t->global_step), ds_idx(t, off));
       }
       SB_CUDA(cudaGetLastError());
       SB_CUDA(cudaEventRecord(t->ev_run_prep[set], t->prep));
@@ -1310,13 +1367,14 @@ int sb_trainer_loss_resident(sb_trainer_t* t, int64_t row_offset, int32_t rows, 
   const bool resident = t->dsXb != nullptr;
   if (resident)
     set_batch_kernel<<<1, 1, 0, n.stream>>>(n.desc, nullptr, t->dsY + row_offset, t->dsW + row_offset, 0.f, 1.f, t->epoch,
-                                             static_cast<int>(row_offset), t->dsP, rows, n.scal);
+                                             static_cast<int>(row_offset), t->dsP, rows, n.scal, nullptr, ds_idx(t, row_offset));
   else
-    set_batch_kernel<<<1, 1, 0, n.stream>>>(n.desc, t->dsX + row_offset * n.F, t->dsY + row_offset, t->dsW + row_offset, 0.f, 1.f,
-                                             t->epoch);
+    set_batch_kernel<<<1, 1, 0, n.stream>>>(n.desc, ds_x(t, row_offset), t->dsY + row_offset, t->dsW + row_offset, 0.f, 1.f,
+                                             t->epoch, 0, nullptr, 0, nullptr, nullptr, ds_idx(t, row_offset));
   SB_CUDA(cudaGetLastError());
-  struct Scope { Net& n; ~Scope() { n.from_resident = false; } } scope{n};
+  struct Scope { Net& n; ~Scope() { n.from_resident = false; n.sparse_step = false; } } scope{n};
   n.from_resident = resident;
+  n.sparse_step = t->ds_sparse;
   if (!resident) SB_TRY(n.enqueue_load(rows));
   SB_TRY(n.enqueue_hidden_forward(rows));
   SB_TRY(n.enqueue_out(rows, true, false, nullptr, nullptr));
@@ -1386,7 +1444,7 @@ int sb_trainer_kernels_per_step(sb_trainer_t* t, int32_t rows) {
   Net& n = t->net;
   BatchDesc* d0 = n.desc; float* s0 = n.scal;
   n.desc = t->descs[0]; n.scal = t->scals[0];      // the graph bakes the pair's pointers
-  const int s = get_graph(t, rows, G_STEP, t->dsXb != nullptr, 0, &ge);
+  const int s = get_graph(t, rows, G_STEP, t->dsXb != nullptr, 0, &ge, t->ds_sparse);
   n.desc = d0; n.scal = s0;
   SB_TRY(s);
   return t->kernels_per_step[rows];
@@ -1407,10 +1465,12 @@ int sb_trainer_profile_step(sb_trainer_t* t, int64_t row_offset, int32_t rows, c
   const bool resident = t->dsXb != nullptr;
   if (resident)
     set_batch_kernel<<<1, 1, 0, n.stream>>>(n.desc, nullptr, t->dsY + row_offset, t->dsW + row_offset, lr_for_step(t, t->global_step),
-                                             gscale, t->epoch, static_cast<int>(row_offset), t->dsP, rows, n.scal);
+                                             gscale, t->epoch, static_cast<int>(row_offset), t->dsP, rows, n.scal, nullptr,
+                                             ds_idx(t, row_offset));
   else
-    set_batch_kernel<<<1, 1, 0, n.stream>>>(n.desc, t->dsX + row_offset * n.F, t->dsY + row_offset, t->dsW + row_offset,
-                                             lr_for_step(t, t->global_step), gscale, t->epoch);
+    set_batch_kernel<<<1, 1, 0, n.stream>>>(n.desc, ds_x(t, row_offset), t->dsY + row_offset, t->dsW + row_offset,
+                                             lr_for_step(t, t->global_step), gscale, t->epoch, 0, nullptr, 0, nullptr, nullptr,
+                                             ds_idx(t, row_offset));
   n.profiling = true;
   n.prof_events.clear(); n.prof_names.clear();
   n.launches = 0;
@@ -1418,6 +1478,7 @@ int sb_trainer_profile_step(sb_trainer_t* t, int64_t row_offset, int32_t rows, c
   int s = SB_OK;
   {
     n.from_resident = resident;
+    n.sparse_step = t->ds_sparse;
     if (resident) s = (cudaMemsetAsync(t->grad, 0, sizeof(float) * n.n_params, n.stream) == cudaSuccess) ? SB_OK : SB_ERR_CUDA;
     n.mark("start"); --n.launches;
     if (!resident) s = n.enqueue_load(rows, t->grad, n.n_params);
@@ -1435,6 +1496,7 @@ int sb_trainer_profile_step(sb_trainer_t* t, int64_t row_offset, int32_t rows, c
   }
   n.profiling = false;
   n.from_resident = false;
+  n.sparse_step = false;
   cudaError_t e = cudaStreamSynchronize(n.stream);
   int cnt = 0;
   std::string joined;

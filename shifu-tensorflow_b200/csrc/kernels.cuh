@@ -18,6 +18,7 @@ struct BatchDesc {
   unsigned int epoch;  // exchange round (flag value of the peer-memory all-reduce)
   int row0;            // first row of the batch inside the bf16 HBM-resident set (TMA row-coordinate offset)
   float2* hist;        // nullable: slot of this step in the pinned-host loss history (loss sum, n_nz), written by the step's tail
+  const int* idx;      // sparse (wide+deep) steps: the batch's index rows [rows, n_cat] - staged, or inside the resident set
 };
 
 // nz_prefix != nullptr (bf16 resident set): the batch is consumed by TMA straight from the resident set, there is no
@@ -25,8 +26,8 @@ struct BatchDesc {
 // and clears the loss accumulator.
 static __global__ void set_batch_kernel(BatchDesc* d, const float* X, const float* y, const float* w, float lr_t, float gscale,
                                         unsigned int epoch = 0, int row0 = 0, const int* nz_prefix = nullptr, int rows = 0,
-                                        float* scal = nullptr, float2* hist = nullptr) {
-  d->X = X; d->y = y; d->w = w; d->lr_t = lr_t; d->gscale = gscale; d->epoch = epoch; d->row0 = row0; d->hist = hist;
+                                        float* scal = nullptr, float2* hist = nullptr, const int* idx = nullptr) {
+  d->X = X; d->y = y; d->w = w; d->lr_t = lr_t; d->gscale = gscale; d->epoch = epoch; d->row0 = row0; d->hist = hist; d->idx = idx;
   if (nz_prefix != nullptr) {
     scal[1] = static_cast<float>(nz_prefix[row0 + rows] - nz_prefix[row0]);  // SCAL_NNZ
     scal[0] = 0.f;                                                           // SCAL_LOSS_SUM
@@ -528,7 +529,8 @@ shadow_refresh_kernel(const OptWork* __restrict__ work, const float* __restrict_
 // ------------------------------------------------------------------------------------------------
 struct EmbedParams {
   int rows, n_cat, H;              // H = width of hidden layer 0
-  const int* idx;                  // [rows, n_cat]
+  const BatchDesc* desc;           // desc->idx = the batch's index rows [rows, n_cat] (read at run time: a captured graph serves
+                                   // any batch)
   const __nv_bfloat16* We;         // bf16 modes: shadow rows of W_e [n_onehot, ldW] (part 0); nullptr in fp32 mode
   long long We_ps; int np;         // parts
   const float* We32;               // fp32 mode: master rows [n_onehot, ldW]
@@ -545,12 +547,13 @@ static __global__ void __launch_bounds__(256) embed_gather_kernel(const EmbedPar
   const int lane = threadIdx.x & 31;
   const int r = blockIdx.x * 8 + (threadIdx.x >> 5);
   if (r >= p.rows) return;
+  const int* __restrict__ idx = p.desc->idx + static_cast<size_t>(r) * p.n_cat;
   for (int c0 = lane * 8; c0 < p.H; c0 += 256) {       // 8 columns per lane per pass
     float acc[8];
 #pragma unroll
     for (int k = 0; k < 8; ++k) acc[k] = 0.f;
     for (int c = 0; c < p.n_cat; ++c) {
-      const int j = __ldg(p.idx + static_cast<size_t>(r) * p.n_cat + c);
+      const int j = __ldg(idx + c);
       if (j < 0) continue;
       if (p.We != nullptr) {
         for (int part = 0; part < p.np; ++part) {
@@ -583,6 +586,7 @@ static __global__ void __launch_bounds__(256) embed_scatter_kernel(const EmbedPa
   const int lane = threadIdx.x & 31;
   const int r = blockIdx.x * 8 + (threadIdx.x >> 5);
   if (r >= p.rows) return;
+  const int* __restrict__ idx = p.desc->idx + static_cast<size_t>(r) * p.n_cat;
   for (int c0 = lane * 4; c0 < p.H; c0 += 128) {       // 4 columns per lane per pass -> red.global.add.v4.f32
     float g[4] = {0.f, 0.f, 0.f, 0.f};
     for (int k = 0; k < 4; ++k) {
@@ -594,7 +598,7 @@ static __global__ void __launch_bounds__(256) embed_scatter_kernel(const EmbedPa
       }
     }
     for (int c = 0; c < p.n_cat; ++c) {
-      const int j = __ldg(p.idx + static_cast<size_t>(r) * p.n_cat + c);
+      const int j = __ldg(idx + c);
       if (j < 0) continue;
       float* dst = p.gWe + static_cast<size_t>(j) * p.H + c0;
       if (c0 + 4 <= p.H && (p.H & 3) == 0 && (reinterpret_cast<uintptr_t>(p.gWe) & 15) == 0) red_add_v4_f32(dst, g[0], g[1], g[2], g[3]);
@@ -603,6 +607,20 @@ static __global__ void __launch_bounds__(256) embed_scatter_kernel(const EmbedPa
           if (c0 + k < p.H) red_add_f32(dst + k, g[k]);
     }
   }
+}
+
+// out[0] = min(out[0], p[0..n)), out[1] = max(out[1], p[0..n)): range check of an index matrix already in device memory
+static __global__ void __launch_bounds__(256) int_range_kernel(const int* __restrict__ p, long long n, int* __restrict__ out) {
+  int lo = 0x7fffffff, hi = -0x7fffffff - 1;
+  for (long long i = blockIdx.x * 256ll + threadIdx.x; i < n; i += gridDim.x * 256ll) {
+    const int v = __ldg(p + i);
+    lo = min(lo, v); hi = max(hi, v);
+  }
+  for (int o = 16; o > 0; o >>= 1) {
+    lo = min(lo, __shfl_xor_sync(0xffffffffu, lo, o));
+    hi = max(hi, __shfl_xor_sync(0xffffffffu, hi, o));
+  }
+  if ((threadIdx.x & 31) == 0) { atomicMin(out, lo); atomicMax(out + 1, hi); }
 }
 
 // acc += g  (epoch-sync schedule: ConditionalAccumulator.apply_grad, res/ssgd_monitor.py:136-141)

@@ -345,7 +345,7 @@ int Net::enqueue_embed(int rows, bool scatter, float* grad, cudaStream_t st) {
   const Layer& l0 = layers[0];
   EmbedParams p = {};
   p.rows = rows; p.n_cat = n_cat; p.H = l0.out;
-  p.idx = idx;
+  p.desc = desc;
   p.np = nparts; p.ldW = tc() ? l0.ld_out : l0.out;
   if (tc()) { p.We = l0.Wn + static_cast<size_t>(n_dense) * l0.ld_out; p.We_ps = Wn_ps[0]; }
   else p.We32 = theta + l0.w_off + static_cast<long long>(n_dense) * l0.out;
@@ -398,6 +398,7 @@ int Net::enqueue_hidden_forward(int rows, float* grad, bool* fused_out) {
     Layer& ly = layers[l];
     if (l == 1 && before_layer1) SB_TRY(before_layer1());
     const bool sp0 = (l == 0) && sparse_step;       // wide+deep: contract the dense columns only, add the embedding sums
+    if (sp0 && from_resident) SB_TRY(enqueue_embed(rows, false, nullptr, stream));   // (no load kernel launched the gather)
     const int k_in = sp0 ? n_dense : ly.in;
     const int ld_k = sp0 ? ldD : ly.ld_in;
     if (tc()) {

@@ -181,7 +181,8 @@ struct Net {
   bool fuse_out_layer = true;
   int fuse_out_max = 256;                    // widest last hidden layer whose GEMM also runs the output layer (one n-tile)
   // bf16 HBM-resident training set (trainer): when `from_resident` is set while enqueueing, layer 0's GEMMs read their A
-  // operand from it by TMA at row offset desc->row0 and no load_batch kernel runs
+  // operand from it by TMA at row offset desc->row0 and no load_batch kernel runs (a sparse step: the set holds the dense
+  // block, pitch ldD, and the embedding gather runs in front of the layer-0 forward GEMM)
   const __nv_bfloat16* resident_Xb = nullptr;
   long long resident_rows = 0;
   bool from_resident = false;

@@ -647,6 +647,7 @@ def main(_=None, env=None, rng=random) -> int:
         if not per_batch_update:
             logging.info("wide+deep trains with one update per mini-batch (Schedule=batch); the sync-replicas accumulator is not wired for sparse steps")
             per_batch_update = True
+        trainer.load_dataset_sparse(train_x, train_idx, train_y, train_w)
     else:
         trainer.load_dataset(train_x, train_y, train_w)
 
@@ -661,13 +662,7 @@ def main(_=None, env=None, rng=random) -> int:
     while trainer.global_step < epochs:           # StopAtStepHook(num_steps=EPOCH) (ssgd_monitor.py:235)
         start = time.time()
         l = 0.0
-        if wide_deep:
-            for i in range(total_batch):
-                a, b = int(bounds[i]), int(bounds[i + 1])
-                l = trainer.step_sparse(train_x[a:b], train_idx[a:b], train_y[a:b], train_w[a:b])
-                if trainer.global_step >= epochs:
-                    break
-        elif per_batch_update:
+        if per_batch_update:
             # the whole `for i in range(total_batch): sess.run(train_step)` loop (ssgd_monitor.py:272-276) as one
             # asynchronous call per run of equally sized batches (np.array_split sizes differ by at most one row)
             for first, count, rows in equal_size_runs(bounds):
