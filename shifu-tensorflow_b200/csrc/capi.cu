@@ -56,7 +56,7 @@ struct sb_trainer {
   P2PPeers* d_peers = nullptr;     // device table of every rank's arena
   std::vector<void*> peer_bases;   // opened IPC mappings (to close)
   bool p2p_ready = false;
-  bool peers_share_device = false; // in-process replicas on this device (tests): see XchgParams::early_dependents
+  bool peers_share_device = false; // in-process replicas on this device (tests): smaller exchange grids, dW_1 behind dW_0
   bool grad_sharded = false;       // the reduced gradient of the last step lives in slices on its owners (sb_trainer_get_grads gathers)
   bool master_stale = false;       // sharded updates ran since the fp32 master / state were last gathered from their owners
   unsigned int epoch = 0;
@@ -73,7 +73,6 @@ struct sb_trainer {
   bool ll_ready = false;           // the LL exchange (xchg_ll_kernel) is usable: plain bf16, world > 1, buffers in the arena
   long long llg_off = 0, lls_off = 0;
   int x_sent = 0;                  // (while enqueueing a step) slots whose exchange the dW_0 chunk hook has launched
-  bool pending_xA = false;         // (while capturing) slot 0's exchange of the previous step has not been joined yet
   // pipelined host-buffer steps (sb_trainer_step_async): second staging slot + copy stream, so the H2D of batch i+1
   // overlaps the compute of batch i
   cudaStream_t copy_stream = nullptr;
@@ -107,14 +106,12 @@ static float lr_for_step(const sb_trainer* t, long long step /*1-based*/) {
   return t->lr;
 }
 
-static int enqueue_allreduce(sb_trainer* t, float* buf, long long off = 0, long long count = -1, cudaStream_t st = nullptr) {
+static int enqueue_allreduce(sb_trainer* t, float* buf) {
   if (t->world <= 1) return SB_OK;
   NcclApi* api = nccl_api();
   SB_CHECK(api && t->comm, SB_ERR_NCCL, "no gradient exchange configured: world = %d but neither an NCCL communicator (nccl_id) nor a "
            "peer table (sb_trainer_set_peer_handles / _pointers) exists", t->world);
-  if (count < 0) count = t->net.n_params;
-  if (!st) st = t->net.stream;
-  int r = api->AllReduce(buf + off, buf + off, static_cast<size_t>(count), NCCL_FLOAT32, NCCL_SUM, t->comm, st);
+  int r = api->AllReduce(buf, buf, static_cast<size_t>(t->net.n_params), NCCL_FLOAT32, NCCL_SUM, t->comm, t->net.stream);
   SB_CHECK(r == 0, SB_ERR_NCCL, "ncclAllReduce failed: %s", api->GetErrorString(r));
   return SB_OK;
 }
@@ -152,22 +149,16 @@ static XchgParams xchg_params(sb_trainer* t) {
   p.hyper = t->hyper;
   p.host_err = t->d_herr;
   p.timeout_ns = t->xchg_timeout_ns;
-  p.early_dependents = 0;
   static const bool fence_sys = getenv("SB_XCHG_FENCE_SYS") != nullptr;
   p.fence_gpu = fence_sys ? 0 : 1;
   return p;
 }
 
 // reduce-scatter -> owner update -> all-gather of the operands for the given segments (xchg_p2p.cuh); `g` must be t->grad
-// release_early: the launch lets its programmatic dependents start as soon as it has started itself (only for a launch whose
-// dependents need nothing it produces, see the deferred slot 0 in enqueue_step_body) - every other launch completes first,
-// also for dependents that were given the programmatic attribute
-static int enqueue_xchg(sb_trainer* t, int slot_mask, cudaStream_t st, bool publish_scalars, bool pdl, bool release_early = false,
-                        bool alone = false) {
+static int enqueue_xchg(sb_trainer* t, int slot_mask, cudaStream_t st, bool publish_scalars, bool pdl, bool alone = false) {
   Net& n = t->net;
   XchgParams p = xchg_params(t);
   p.slot_mask = slot_mask;
-  p.early_dependents = (release_early && !t->peers_share_device) ? 1 : 0;
   p.scal = publish_scalars ? n.scal : nullptr;
   p.host_scal = publish_scalars ? t->d_hscal : nullptr;
   char nm[24];
@@ -192,15 +183,10 @@ static int enqueue_xchg(sb_trainer* t, int slot_mask, cudaStream_t st, bool publ
   if (grid > want) grid = want;
   if (grid < 1) grid = 1;
   const dim3 g(static_cast<unsigned>(grid)), b(256);
-  // SB_XCHG_LL = all (default) | last | none: which launches use the LL protocol (flags inside the data).  Measured on 2 x B200,
-  // cfg2: all 163.8 us/step, last (only the launch nothing runs beside) 168.2, none 171.4; an LL launch takes 21-28 us where
+  // Every launch uses the LL protocol (flags inside the data) where it is available.  Measured on 2 x B200, cfg2: LL for every
+  // launch 163.8 us/step, only for the launch nothing runs beside 168.2, for none 171.4; an LL launch takes 21-28 us where
   // the flag-and-pull kernel takes 32-47, at the price of 2-4 us on the GEMM beside it (polling, doubled store traffic).
-  static const int ll_mode = [] {
-    const char* e = getenv("SB_XCHG_LL");
-    if (e == nullptr) return 2;
-    return strcmp(e, "last") == 0 ? 1 : (strcmp(e, "none") == 0 ? 0 : 2);
-  }();
-  if (t->ll_ready && (ll_mode == 2 || (ll_mode == 1 && alone))) {
+  if (t->ll_ready) {
     LLParams lp;
     lp.x = p; lp.llg_off = t->llg_off; lp.lls_off = t->lls_off; lp.n4 = t->xch_n4;
     if (t->world <= 2) SB_TRY(n.launch(xchg_ll_kernel<2>, g, b, 0, st, pdl, lp));
@@ -231,69 +217,44 @@ static int gather_master(sb_trainer* t) {
   return SB_OK;
 }
 
-// SB_PIPELINE_AR=1 (opt-in): per-layer exchange + update on the comm stream; then no single tail kernel exists and the
-// step scalars are read back with a copy instead
-static bool step_is_pipelined(const sb_trainer* t, int kind) {
-  static const bool want_pipeline = getenv("SB_PIPELINE_AR") != nullptr;
-  const Net& n = t->net;
-  return want_pipeline && kind == G_STEP && n.concurrent_bwd && !n.profiling && n.side != nullptr &&
-         n.tc();
-}
-
 // the body of one step as a sequence of stream operations (captured into a CUDA graph)
-static int enqueue_step_body(sb_trainer* t, int rows, int kind, bool resident = false, bool sparse = false, bool last_in_graph = true) {
+static int enqueue_step_body(sb_trainer* t, int rows, int kind, bool resident = false, bool sparse = false) {
   Net& n = t->net;
   struct Scope {
     Net& n;
     ~Scope() {
       n.from_resident = false; n.zero_buf = nullptr; n.dw0_on_main = n.defer_join = false; n.sparse_step = false;
-      n.dw0_chunks = 1; n.dw1_last = false; n.on_dw0_chunk = nullptr; n.before_layer1 = nullptr; n.zero_layer = 0;
+      n.dw0_chunks = 1; n.dw1_last = false; n.on_dw0_chunk = nullptr;
       n.dw1_first = false; n.after_dw1 = nullptr; n.dw1_serial_auto = false;
-      n.beside_prev_xchg = false;
     }
   } scope{n};
   n.from_resident = resident;
   n.sparse_step = sparse;
   n.trace_k = 0;
-  // ---- schedule of the step's tail (decided first: the peer-exchange schedule also changes the forward pass) ----
-  const bool pipelined = step_is_pipelined(t, kind);
+  // ---- schedule of the step's tail ----
   // Single GPU, one update per mini-batch: no exchange, so nothing needs ALL gradients at once.  dW_0 runs on the main
   // stream behind the last dA GEMM and is followed (PDL) by the optimizer of layer 0 alone; the side stream updates the
   // other layers right after their dW GEMMs; the two streams only join at the end of the graph.
-  static const bool old_sched = getenv("SB_OLD_SCHED") != nullptr;
-  static const bool one_xchg = getenv("SB_XCHG_ONE") != nullptr;    // experiment: one exchange launch for everything after a join
-  const bool split_tail = !old_sched && kind == G_STEP && (t->world == 1 || (t->p2p_ready && !one_xchg)) && !pipelined &&
-                          n.concurrent_bwd && !n.profiling && n.side != nullptr && n.tc() && n.L > 1;
+  const bool split_tail = kind == G_STEP && (t->world == 1 || t->p2p_ready) && !n.profiling && n.side != nullptr && n.tc() &&
+                          n.L > 1;
   // Peer exchange (world > 1): one exchange launch costs 20-30 us through NVSwitch however little data it moves (fabric latency,
-  // xchg_p2p.cuh) - hidden when a GEMM follows it, exposed in full behind the last GEMM.  Default order ("first"):
+  // xchg_p2p.cuh) - hidden when a GEMM follows it, exposed in full behind the last GEMM:
   //   main:  ... dA_1 -> dW_1 -> dW_0 chunk 0 -> dW_0 chunk 1 | wait A, B0, B1 | next step
   //   side:  ... dW_2 ...     A ------------->
   //   comm:                             B0 ---------------->    B1 ------>
-  // A (every layer but hidden layer 0) and B0 run beside dW_0's chunks, only B1 - half of layer 0 - is exposed.
-  // Order "last" (SB_XCHG_ORDER=last, and replicas that share a device): dW_1 BEHIND dW_0 as cover for B1, and A beside the
-  // NEXT step's layer-0 forward GEMM, which reads nothing slot A writes: layer 1's forward waits for A, and - because peers
-  // may read this rank's gradient buffer until then - the buffer is cleared by layer 1's forward GEMM instead of layer 0's.
+  // dW_1 runs in front of dW_0: A (every layer but hidden layer 0) and B0 hide behind dW_0's chunks, only B1 - half of layer
+  // 0 - runs on an otherwise idle GPU (an exchange kernel beside a GEMM takes 40-47 us, alone ~25; measured, 2 x B200).
+  // Replicas that share ONE device (tests) put dW_1 BEHIND dW_0 as cover for B1, and A behind dW_1: with three exchange
+  // launches of both replicas waiting beside each other's persistent GEMMs the order above stopped making progress within
+  // the exchange timeout.
   const bool xsched = split_tail && t->world > 1;
-  // SB_XCHG_ORDER: "first" (default) = dW_1 in front of dW_0: slot A and chunk 0 hide behind dW_0's chunks, the LAST chunk's
-  // exchange runs on an otherwise idle GPU - an exchange kernel beside a GEMM takes 40-47 us, alone ~25 (measured, 2 x B200);
-  // "last" = dW_1 behind dW_0 as cover for the last chunk, slot A beside the next step's layer-0 forward.
-  static const bool order_last_env = getenv("SB_XCHG_ORDER") != nullptr && strcmp(getenv("SB_XCHG_ORDER"), "last") == 0;
-  // (replicas that share ONE device - tests - keep the "last" order: with three exchange launches of both replicas waiting
-  // beside each other's persistent GEMMs the "first" order stopped making progress within the exchange timeout)
-  const bool order_last = order_last_env || t->peers_share_device;
-  static const bool no_defer = getenv("SB_XCHG_NO_DEFER") != nullptr;
-  // (not for sparse steps: the embedding gather in front of the layer-0 forward GEMM would let it skip a wait it needs)
-  const bool defer_A = xsched && order_last && resident && n.L >= 3 && !no_defer && !sparse;
-  if (xsched) {
-    n.zero_layer = defer_A ? 1 : 0;
-    n.beside_prev_xchg = t->pending_xA;     // slot A's exchange of the previous step is the kernel in front of this step
-    t->pending_xA = false;
-  }
+  const bool order_last = t->peers_share_device;
   if (resident) {
     // no load kernel: the batch is read by TMA from the bf16 resident set; set_batch_kernel already published n_nz.
     // The gradient buffer is first written by the last forward layer's epilogue, so with more than one hidden layer the
     // layer-0 forward GEMM clears it (its epilogue warps idle until their first accumulator completes); a memset node
-    // at the head of the chain cost ~3 us per step.
+    // at the head of the chain cost ~3 us per step.  No peer reads it any more: the previous step's main stream waited
+    // for every exchange.
     if (n.L > 1) {
       n.zero_buf = reinterpret_cast<float4*>(t->grad);   // cudaMalloc'ed, padded to xch_n4 float4
       n.zero_n4 = t->xch_n4;
@@ -306,46 +267,17 @@ static int enqueue_step_body(sb_trainer* t, int rows, int kind, bool resident = 
   bool fused_out = false;
   SB_TRY(n.enqueue_hidden_forward(rows, t->grad, &fused_out));
   if (!fused_out) SB_TRY(n.enqueue_out(rows, true, true, nullptr, t->grad));
-  // Gradient exchange pipelined behind the backward pass: as soon as layer l's dW GEMM is enqueued (side stream), its
-  // flat segment [W_l, b_l] (+ the output layer for l = L-1) is all-reduced and its optimizer update applied on the
-  // comm stream while the remaining dA / dW GEMMs still run - the role SyncReplicasOptimizer's accumulator + apply
-  // play in the reference (res/ssgd_monitor.py:136-142), without the parameter server.
-  // Measured on 2x B200 (profiles/scaling_r01.md): with NCCL as the exchange, ONE all-reduce of the whole flat gradient
-  // after the backward pass beats per-layer / per-chunk calls (each NCCL launch costs ~20-50 us and its CTAs evict
-  // persistent GEMM CTAs), so the pipelined variant is opt-in (SB_PIPELINE_AR=1).
-  if (pipelined) {
-    n.on_layer_grads = [t](int l, cudaStream_t cs, int phase, long long e0, long long e1) -> int {
-      Net& nn = t->net;
-      const Layer& ly = nn.layers[l];
-      const int last = (l == nn.L - 1) ? nn.L : l;
-      const bool completes = e1 == static_cast<long long>(ly.in) * ly.out;  // this chunk also carries b_l (+ output layer)
-      if (phase == 0) {
-        const long long off = ly.w_off + e0;
-        const long long end = completes ? nn.layers[last].b_off + nn.layers[last].out : ly.w_off + e1;
-        return enqueue_allreduce(t, t->grad, off, end - off, cs);
-      }
-      // work-table runs are 1024 parameters each, chunk boundaries are multiples of 1024 (128 rows x out % 8 == 0)
-      const int w0 = nn.work_begin[l] + static_cast<int>(e0 / 1024);
-      const int w1 = completes ? nn.work_end[last] : nn.work_begin[l] + static_cast<int>(e1 / 1024);
-      return enqueue_optimizer(t, t->grad, w0, w1, cs);
-    };
-  } else {
-    n.on_layer_grads = nullptr;
-  }
   // (dW_0 on the main stream also when an exchange or the accumulate kernel follows: it is then joined with the side
   // stream as before)
-  n.dw0_on_main = !old_sched && !pipelined && n.concurrent_bwd && !n.profiling && n.side != nullptr &&
-                  n.tc() && n.L > 1;
+  n.dw0_on_main = !n.profiling && n.side != nullptr && n.tc() && n.L > 1;
   n.defer_join = split_tail;
   cudaStream_t comms[2] = {n.comm2, n.comm};
   if (xsched) {
-    // dW_1 leaves the side stream: in front of dW_0 ("first") or behind it ("last").  (SB_XCHG_BESIDE=1 keeps it beside dW_0
-    // like the single-GPU schedule; measured on 2 x B200: the chunks of dW_0 then share the SMs with dW_1 - 31 + 19 us
-    // instead of 18 + 19.)
-    static const bool beside = getenv("SB_XCHG_BESIDE") != nullptr;
+    // dW_1 leaves the side stream.  (Beside dW_0, like the single-GPU schedule, the chunks of dW_0 shared the SMs with dW_1:
+    // 31 + 19 us instead of 18 + 19, measured on 2 x B200.)
     n.dw0_chunks = t->x_chunks;
-    n.dw1_last = !beside && order_last;
-    n.dw1_first = !beside && !order_last;
+    n.dw1_last = order_last;
+    n.dw1_first = !order_last;
     t->x_sent = 0;
     if (n.dw1_first) {
       n.after_dw1 = [t]() -> int {       // slot A on the side stream, behind dW_1 (main) and the other layers' dW GEMMs (side)
@@ -364,15 +296,14 @@ static int enqueue_step_body(sb_trainer* t, int rows, int kind, bool resident = 
       SB_CUDA(cudaEventRecord(t->ev_c[1 + c], nn.stream));
       SB_CUDA(cudaStreamWaitEvent(cs, t->ev_c[1 + c], 0));
       const bool last = c == t->x_chunks - 1;
-      SB_TRY(enqueue_xchg(t, 1 << (1 + c), cs, last, false, false, last && !nn.dw1_last));   // (the last chunk publishes the step scalars;
-                                                                                              //  no GEMM follows it unless dW_1 does)
+      SB_TRY(enqueue_xchg(t, 1 << (1 + c), cs, last, false, last && !nn.dw1_last));   // (the last chunk publishes the step scalars;
+                                                                                      //  no GEMM follows it unless dW_1 does)
       SB_CUDA(cudaEventRecord(t->ev_x[1 + c], cs));
       t->x_sent |= 1 << (1 + c);
       return SB_OK;
     };
   }
-  static const bool dw1_beside_n1 = getenv("SB_DW1_BESIDE") != nullptr;
-  if (split_tail && !xsched && !dw1_beside_n1) {
+  if (split_tail && !xsched) {
     // one GPU: dW_1 may move in front of dW_0 (Net::dw1_serial_auto); the side stream's optimizer launch then waits for it
     n.dw1_serial_auto = true;
     n.after_dw1 = [t]() -> int {
@@ -382,48 +313,29 @@ static int enqueue_step_body(sb_trainer* t, int rows, int kind, bool resident = 
       return SB_OK;
     };
   }
-  int bs = n.enqueue_backward(rows, t->grad);
-  n.on_layer_grads = nullptr;
-  SB_TRY(bs);
+  SB_TRY(n.enqueue_backward(rows, t->grad));
   if (xsched) {
     // slot A: every gradient but hidden layer 0's - complete behind dW_1 (main stream), the other layers' dW GEMMs (side
-    // stream) and the last dA GEMM (the last reader of their weight shadows).
-    // Deferred (multi-step graphs): the launch goes ON the main stream, as dW_1's programmatic dependent.  It releases ITS
-    // dependents at its start, the next step's layer-0 forward GEMM skips its dependency wait (all it needs - B0, B1 - are
-    // full dependencies) and so runs beside the exchange; layer 1's forward is a plain in-stream launch behind both.
-    // (As a node on another stream that nothing on the main chain waited for, the graph executor started the exchange 18 us
-    // after B1 had ENDED - whichever stream carried it, with or without a waited-for marker kernel in front.)
-    const bool a_on_main = defer_A && n.dw1_last && !t->peers_share_device;
-    if (t->x_sent & XSEG_A) {
-      // (dW_1 first: launched by after_dw1)
-    } else if (a_on_main) {
-      if (n.L > 2) {
-        SB_CUDA(cudaEventRecord(n.ev_join, n.side));
-        SB_CUDA(cudaStreamWaitEvent(n.stream, n.ev_join, 0));
-      }
-      SB_TRY(enqueue_xchg(t, XSEG_A, n.stream, false, n.use_pdl, !last_in_graph));
-    } else {
-      if (n.dw1_last) {
-        SB_CUDA(cudaEventRecord(t->ev_c[0], n.stream));
-        SB_CUDA(cudaStreamWaitEvent(n.side, t->ev_c[0], 0));
-      } else {
-        SB_CUDA(cudaStreamWaitEvent(n.side, n.ev_da_done, 0));
-      }
+    // stream) and the last dA GEMM (the last reader of their weight shadows).  With dW_1 in front of dW_0, after_dw1 has
+    // launched it; with dW_1 behind dW_0 it goes to the side stream here.
+    if (!(t->x_sent & XSEG_A)) {
+      SB_CUDA(cudaEventRecord(t->ev_c[0], n.stream));
+      SB_CUDA(cudaStreamWaitEvent(n.side, t->ev_c[0], 0));
       SB_TRY(enqueue_xchg(t, XSEG_A, n.side, false, false));
       SB_CUDA(cudaEventRecord(t->ev_x[0], n.side));
     }
-    // whatever follows on the main stream (the next step's layer-0 forward, or the end of the graph) needs hidden layer 0
+    // whatever follows on the main stream (the next step, which clears the gradient buffer peers read, or the end of the
+    // graph) waits for every slot
     for (int c = 0; c < t->x_chunks; ++c)
       if ((t->x_sent >> (1 + c)) & 1) SB_CUDA(cudaStreamWaitEvent(n.stream, t->ev_x[1 + c], 0));
     // (a layer-0 dW that was not cut into the trainer's chunks - wide+deep steps - is exchanged here, behind everything)
     const int missing = (xseg_all(t) & ~XSEG_A) & ~t->x_sent;
     if (missing) SB_TRY(enqueue_xchg(t, missing, n.stream, true, false));
-    if (a_on_main) t->pending_xA = !last_in_graph;      // (the last step of a graph: whatever follows is ordered behind it)
-    else SB_CUDA(cudaStreamWaitEvent(n.stream, t->ev_x[0], 0));
+    SB_CUDA(cudaStreamWaitEvent(n.stream, t->ev_x[0], 0));
     return SB_OK;
   }
   if (split_tail) {
-    SB_TRY(enqueue_optimizer(t, t->grad, n.work_begin[0], n.work_end[0], n.stream, true, n.use_pdl));
+    SB_TRY(enqueue_optimizer(t, t->grad, n.work_begin[0], n.work_end[0], n.stream, true, true));
     // the other layers' shadows are read by the dA GEMMs on the main stream: update them only after the last one
     SB_CUDA(cudaStreamWaitEvent(n.side, n.ev_da_done, 0));
     SB_TRY(enqueue_optimizer(t, t->grad, n.work_end[0], n.n_work, n.side));
@@ -432,9 +344,8 @@ static int enqueue_step_body(sb_trainer* t, int rows, int kind, bool resident = 
     return SB_OK;
   }
   if (kind == G_STEP) {
-    if (pipelined) return SB_OK;
     if (t->world > 1 && t->p2p_ready) {
-      // (fp32 mode, one hidden layer, profiling, SB_XCHG_ONE: no split tail) one launch handles both segments
+      // (fp32 mode, one hidden layer: no split tail) one launch handles both segments
       SB_TRY(enqueue_xchg(t, xseg_all(t), n.stream, true, false));
     } else {
       SB_TRY(enqueue_allreduce(t, t->grad));
@@ -480,8 +391,7 @@ static int run_step(sb_trainer* t, const float* X, const float* y, const float* 
   static const bool no_graph = getenv("SB_NO_GRAPH") != nullptr;
   const bool resident = resident_row0 >= 0 && t->dsXb != nullptr;
   // descriptor / scalar pair of this step: resident graph steps alternate, everything else uses pair 0
-  static const bool want_prep = !(getenv("SB_PREP") && getenv("SB_PREP")[0] == '0');
-  const bool prep = want_prep && resident && !no_graph && t->prep != nullptr;
+  const bool prep = resident && !no_graph;
   const int pair = prep ? static_cast<int>(t->prep_steps & 1) : 0;
   n.desc = t->descs[pair];
   n.scal = t->scals[pair];
@@ -520,8 +430,6 @@ static int run_step(sb_trainer* t, const float* X, const float* y, const float* 
   if (no_graph) SB_TRY(enqueue_step_body(t, rows, kind, resident, sparse));
   else SB_CUDA(cudaGraphLaunch(ge, n.stream));
   // the step's tail kernel (optimizer / accumulate) wrote (loss sum, n_nz) into h_scal; visible after a stream sync
-  if (step_is_pipelined(t, kind))
-    SB_CUDA(cudaMemcpyAsync(t->h_scal, n.scal, sizeof(float) * SCAL_COUNT, cudaMemcpyDeviceToHost, n.stream));
   if (kind == G_ACC) ++t->n_acc;
   t->grad_out_scale = (kind == G_STEP) ? gscale : 1.f;
   return SB_OK;
@@ -637,19 +545,17 @@ int sb_trainer_create(const sb_net_desc* desc, int device, const void* nccl_id, 
     t->xch_n4 = (np + 3) / 4;
     t->net.arena_extra_bytes = static_cast<size_t>(t->xch_n4) * 16 + sizeof(P2PFlags);
     // LL exchange buffers (xchg_p2p.cuh): gbuf = world regions, sbuf = one, of n4 entries x 32 bytes
-    static const bool no_ll = getenv("SB_XCHG_PULL") != nullptr;
-    if (world > 1 && desc->precision == SB_PREC_BF16 && !no_ll) {
+    if (world > 1 && desc->precision == SB_PREC_BF16) {
       t->ll_ready = true;
       t->net.arena_extra_bytes += 256 + static_cast<size_t>(world + 1) * static_cast<size_t>(t->xch_n4) * 32;
     }
   }
   int s = t->net.init(desc, device, true);
   if (s != SB_OK) { t->net.destroy(); return s; }
-  if (!getenv("SB_NO_CARVEOUT")) {   // see Net::init: no L1 / shared-memory re-partition between the kernels of a step
-    cudaFuncSetAttribute(set_batch_kernel, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared);
-    cudaFuncSetAttribute(optimizer_kernel, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared);
-    cudaFuncSetAttribute(axpy_kernel, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared);
-  }
+  // see Net::init: no L1 / shared-memory re-partition between the kernels of a step
+  cudaFuncSetAttribute(set_batch_kernel, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared);
+  cudaFuncSetAttribute(optimizer_kernel, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared);
+  cudaFuncSetAttribute(axpy_kernel, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared);
   Net& n = t->net;
   // gradient + exchange flags behind the parameters, in the arena a single IPC handle exports
   t->xch = n.arena;
@@ -731,22 +637,6 @@ int sb_trainer_create(const sb_net_desc* desc, int device, const void* nccl_id, 
     return set_error(SB_ERR_CUDA, "cudaHostGetDevicePointer failed");
   }
   if (world > 1 && nccl_id != nullptr) {
-    // The GEMMs are persistent (one CTA per SM, ~200 KB smem each): an NCCL CTA that lands on an SM evicts a GEMM CTA
-    // into a second wave.  Keep NCCL to a few CTAs and leave those SMs out of the GEMM grids.
-    // (only when the exchange is pipelined behind the backward pass, SB_PIPELINE_AR=1)
-    if (getenv("SB_PIPELINE_AR")) {
-      int nccl_ctas = 8;
-      if (const char* e = getenv("SB_NCCL_CTAS")) nccl_ctas = atoi(e);
-      if (nccl_ctas < 1) nccl_ctas = 1;
-      if (nccl_ctas > 32) nccl_ctas = 32;
-      char buf[16];
-      snprintf(buf, sizeof(buf), "%d", nccl_ctas);
-      setenv("NCCL_MAX_CTAS", buf, 0);
-      n.gemm_sms = n.num_sms - nccl_ctas;
-      n.gemm_sms -= n.gemm_sms & 1;  // CTA pairs
-      n.dw_chunk_bytes = 2500000;
-      if (const char* e = getenv("SB_DW_CHUNK_BYTES")) n.dw_chunk_bytes = atoll(e);
-    }
     NcclApi* api = nccl_api();
     if (!api) { n.destroy(); return set_error(SB_ERR_NCCL, "libnccl.so.2 could not be loaded"); }
     NcclUniqueId id;
@@ -1262,17 +1152,15 @@ static int get_run_graph(sb_trainer* t, int rows, int set, cudaGraphExec_t* out)
   cudaGraph_t g = nullptr;
   SB_CUDA(cudaStreamBeginCapture(n.stream, cudaStreamCaptureModeThreadLocal));
   int s = SB_OK;
-  t->pending_xA = false;
   for (int k = 0; k < sb_trainer::RUN_S && s == SB_OK; ++k) {
     n.desc = t->run_descs[set][k];
     n.scal = t->run_scals[set][k];
-    // (SB_STEP_TRACE: an interior step is the one traced - with the peer exchange, the last step of a graph joins the
-    // exchange of slot A at its end instead of hiding it behind the next step's layer-0 forward)
+    // (SB_STEP_TRACE: the trace holds one step; an interior one is traced, with steps of the same graph on both sides of
+    // it like most steps of a run)
     n.trace_on = (k == 1);
-    s = enqueue_step_body(t, rows, G_STEP, true, t->ds_sparse, k == sb_trainer::RUN_S - 1);
+    s = enqueue_step_body(t, rows, G_STEP, true, t->ds_sparse);
   }
   n.trace_on = true;
-  t->pending_xA = false;
   n.desc = d0; n.scal = s0;
   cudaError_t e = cudaStreamEndCapture(n.stream, &g);
   if (s != SB_OK) { if (g) cudaGraphDestroy(g); return s; }
@@ -1299,7 +1187,7 @@ int sb_trainer_run_resident(sb_trainer_t* t, const int64_t* row_offsets, int32_t
   static const bool no_graph = getenv("SB_NO_GRAPH") != nullptr;
   static const bool no_multi = getenv("SB_NO_MULTI_STEP") != nullptr;
   int i = 0;
-  if (t->dsXb != nullptr && t->prep != nullptr && !no_graph && !no_multi) {
+  if (t->dsXb != nullptr && !no_graph && !no_multi) {
     SB_CUDA(cudaSetDevice(n.device));
     if (t->run_descs[0][0] == nullptr) {
       for (int set = 0; set < 2; ++set) {

@@ -47,8 +47,6 @@ struct GemmTcParams {
   int M, N, K;
   int kb_per_split;  // k-blocks (of 64) per split
   int split_k;       // number of splits actually used (all non-empty)
-  int no_dep_wait;   // 1: do not wait for the programmatic primary (an exchange kernel this GEMM may run beside, capi.cu);
-                     // every real dependency of the launch is then a full one
   // EPI_FWD
   const float* bias;  // [N]
   int act;            // FWD: activation applied; DA: activation whose derivative is applied
@@ -217,7 +215,7 @@ gemm_tc_kernel(const __grid_constant__ TmapSet tms, const GemmTcParams p) {
   // PDL: everything above (barrier init, TMEM allocation, descriptor prefetch) overlapped the previous kernel's tail;
   // from here on global memory written by it is touched.
   if (threadIdx.x == 0) stamp(1);  // setup done
-  if (!p.no_dep_wait) pdl_wait();
+  pdl_wait();
   pdl_launch_dependents();
   if (threadIdx.x == 0) stamp(2);  // dependencies resolved
 

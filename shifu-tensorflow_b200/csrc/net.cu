@@ -148,17 +148,11 @@ int Net::init(const sb_net_desc* d, int device_, bool training_) {
   SB_TRY(check_device(device_, &num_sms));
   device = device_;
   training = training_;
-  if (const char* e = getenv("SB_NO_PDL")) use_pdl = !(e[0] == '1');
-  if (const char* e = getenv("SB_NO_FORK")) concurrent_bwd = !(e[0] == '1');
-  if (const char* e = getenv("SB_NO_FUSE_OUT")) fuse_out_layer = !(e[0] == '1');
-  if (const char* e = getenv("SB_FUSE_OUT_MAX")) fuse_out_max = atoi(e);   // experiment: 128 restores the round-1 rule
   const bool want_trace = getenv("SB_STEP_TRACE") != nullptr;
-  gemm_sms = num_sms;
   SB_CUDA(cudaSetDevice(device));
   // the main chain is the critical path: its CTAs are scheduled ahead of the side stream's (dW GEMMs, second optimizer)
   int prio_least = 0, prio_greatest = 0;
   SB_CUDA(cudaDeviceGetStreamPriorityRange(&prio_least, &prio_greatest));
-  if (getenv("SB_FLAT_PRIO")) prio_greatest = prio_least;      // experiment: every stream at the same priority
   SB_CUDA(cudaStreamCreateWithPriority(&stream, cudaStreamNonBlocking, prio_greatest));
   if (training_) {
     SB_CUDA(cudaStreamCreateWithPriority(&side, cudaStreamNonBlocking, prio_least));
@@ -168,11 +162,6 @@ int Net::init(const sb_net_desc* d, int device_, bool training_) {
     SB_CUDA(cudaEventCreateWithFlags(&ev_da_done, cudaEventDisableTiming));
     SB_CUDA(cudaStreamCreateWithFlags(&comm, cudaStreamNonBlocking));
     SB_CUDA(cudaStreamCreateWithFlags(&comm2, cudaStreamNonBlocking));
-    ev_dw.resize(d->n_hidden);
-    for (auto& e : ev_dw) SB_CUDA(cudaEventCreateWithFlags(&e, cudaEventDisableTiming));
-    ev_da.resize(d->n_hidden);
-    for (auto& e : ev_da) SB_CUDA(cudaEventCreateWithFlags(&e, cudaEventDisableTiming));
-    SB_CUDA(cudaEventCreateWithFlags(&ev_comm, cudaEventDisableTiming));
   }
   F = d->n_features;
   L = d->n_hidden;
@@ -292,12 +281,10 @@ int Net::init(const sb_net_desc* d, int device_, bool training_) {
     SB_TRY((set_gemm_tc_attrs<EPI_DA, false, false>()));
     SB_TRY((set_gemm_tc_attrs<EPI_DW, true, true>()));
     // keep the SMs in the GEMMs' shared-memory carve-out for every kernel of the step, so that no launch in the chain
-    // has to re-partition L1 / shared memory (experiment: SB_NO_CARVEOUT=1 restores the defaults)
-    if (!getenv("SB_NO_CARVEOUT")) {
-      const int co = cudaSharedmemCarveoutMaxShared;
-      cudaFuncSetAttribute(load_batch_kernel<true>, cudaFuncAttributePreferredSharedMemoryCarveout, co);
-      cudaFuncSetAttribute(out_layer_kernel<__nv_bfloat16>, cudaFuncAttributePreferredSharedMemoryCarveout, co);
-    }
+    // has to re-partition L1 / shared memory
+    const int co = cudaSharedmemCarveoutMaxShared;
+    cudaFuncSetAttribute(load_batch_kernel<true>, cudaFuncAttributePreferredSharedMemoryCarveout, co);
+    cudaFuncSetAttribute(out_layer_kernel<__nv_bfloat16>, cudaFuncAttributePreferredSharedMemoryCarveout, co);
   }
   return SB_OK;
 }
@@ -312,12 +299,6 @@ void Net::destroy() {
   ev_join = nullptr;
   if (ev_da_done) cudaEventDestroy(ev_da_done);
   ev_da_done = nullptr;
-  for (cudaEvent_t e : ev_dw) cudaEventDestroy(e);
-  ev_dw.clear();
-  for (cudaEvent_t e : ev_da) cudaEventDestroy(e);
-  ev_da.clear();
-  if (ev_comm) cudaEventDestroy(ev_comm);
-  ev_comm = nullptr;
   if (comm) cudaStreamDestroy(comm);
   comm = nullptr;
   if (comm2) cudaStreamDestroy(comm2);
@@ -380,11 +361,11 @@ int Net::enqueue_load(int rows, float* zero_buf, long long zero_n) {
   if (blocks < 1) blocks = 1;
   // first kernel of the step: its stream predecessor is set_batch_kernel (a kernel), so PDL applies here too
   if (tc())
-    SB_TRY(launch(load_batch_kernel<true>, dim3(static_cast<unsigned>(blocks)), dim3(256), 0, stream, use_pdl,
+    SB_TRY(launch(load_batch_kernel<true>, dim3(static_cast<unsigned>(blocks)), dim3(256), 0, stream, true,
                   static_cast<const BatchDesc*>(desc), rows, Fx, Xb, ldx, static_cast<float*>(nullptr), scal, zero_buf, zero_n,
                   nparts, Xb_ps));
   else
-    SB_TRY(launch(load_batch_kernel<false>, dim3(static_cast<unsigned>(blocks)), dim3(256), 0, stream, use_pdl,
+    SB_TRY(launch(load_batch_kernel<false>, dim3(static_cast<unsigned>(blocks)), dim3(256), 0, stream, true,
                   static_cast<const BatchDesc*>(desc), rows, Fx, static_cast<__nv_bfloat16*>(nullptr), ldx, Xf, scal, zero_buf, zero_n,
                   1, 0ll));
   mark("load_batch");
@@ -396,14 +377,13 @@ int Net::enqueue_hidden_forward(int rows, float* grad, bool* fused_out) {
   if (fused_out) *fused_out = false;
   for (int l = 0; l < L; ++l) {
     Layer& ly = layers[l];
-    if (l == 1 && before_layer1) SB_TRY(before_layer1());
     const bool sp0 = (l == 0) && sparse_step;       // wide+deep: contract the dense columns only, add the embedding sums
     if (sp0 && from_resident) SB_TRY(enqueue_embed(rows, false, nullptr, stream));   // (no load kernel launched the gather)
     const int k_in = sp0 ? n_dense : ly.in;
     const int ld_k = sp0 ? ldD : ly.ld_in;
     if (tc()) {
       // Z = A_{l-1}[rows,in] (K-major) x W_l[in,out] (MN-major B operand: n contiguous)
-      const GemmPlan pl = plan_gemm(rows, ly.out, round_up(k_in, 64) * pairs_of(nparts), gemm_sms, false);
+      const GemmPlan pl = plan_gemm(rows, ly.out, round_up(k_in, 64) * pairs_of(nparts), num_sms, false);
       TmapSet tm;
       const bool res0 = (l == 0) && from_resident;
       const __nv_bfloat16* src = (l == 0) ? (res0 ? resident_Xb : Xb) : A[l - 1];
@@ -417,7 +397,7 @@ int Net::enqueue_hidden_forward(int rows, float* grad, bool* fused_out) {
       p.bias = theta + ly.b_off; p.act = ly.act;
       p.out = A[l]; p.ld_out = ly.ld_out; p.out_ps = A_ps[l];
       p.a_rows = res0 ? desc : nullptr;
-      if (l == L - 1 && grad != nullptr && fuse_out_layer && training && ly.out <= fuse_out_max) {
+      if (l == L - 1 && grad != nullptr && training && ly.out <= fuse_out_max) {
         // K2 + K3 + K4 + output backward in one kernel: one n-tile must cover the whole layer width
         GemmPlan fp = pl;
         fp.split_k = 1; fp.kb_per_split = ((k_in + 63) / 64) * pairs_of(nparts);
@@ -426,7 +406,7 @@ int Net::enqueue_hidden_forward(int rows, float* grad, bool* fused_out) {
         if (ly.out <= 64) { fp.cg = 1; fp.bn = 64; }
         else if (ly.out <= 128) { fp.cg = 1; fp.bn = 128; }
         else { fp.cg = 1; fp.bn = 256; }
-        const int slots = gemm_sms / fp.cg;
+        const int slots = num_sms / fp.cg;
         const int tiles = (rows + 128 * fp.cg - 1) / (128 * fp.cg);
         fp.grid = (tiles < slots ? tiles : slots) * fp.cg;
         Layer& ol = layers[L];
@@ -435,20 +415,19 @@ int Net::enqueue_hidden_forward(int rows, float* grad, bool* fused_out) {
         p.desc = desc; p.scal = scal; p.loss = loss;
         p.g_wo = grad + ol.w_off; p.g_bo = grad + ol.b_off; p.g_bL = grad + ly.b_off;
         p.trace = next_trace("fwd_out", l, rows, ly.out, k_in);
-        SB_TRY((launch_gemm_tc<EPI_FWD_OUT, false, true>(fp, tm, p, stream, use_pdl)));
+        SB_TRY((launch_gemm_tc<EPI_FWD_OUT, false, true>(fp, tm, p, stream, true)));
         if (fused_out) *fused_out = true;
         mark("gemm_fwd_out");
         continue;
       }
-      if (l == zero_layer && zero_buf != nullptr) {
+      if (l == 0 && zero_buf != nullptr) {
         p.zero_buf = zero_buf; p.zero_n4 = zero_n4;
         zero_buf = nullptr;
       }
       p.trace = next_trace("fwd", l, rows, ly.out, k_in);
       if (nparts == 1 && p.addend == nullptr)      // plain bf16: the epilogue stores its tiles by TMA
         SB_TRY(make_tmap_bf16(&tm.o, A[l], rows, ly.out, ly.ld_out, 128));
-      if (beside_prev_xchg && l == 0) p.no_dep_wait = 1;
-      SB_TRY((launch_gemm_tc<EPI_FWD, false, true>(pl, tm, p, stream, use_pdl && !(beside_prev_xchg && l == 1))));
+      SB_TRY((launch_gemm_tc<EPI_FWD, false, true>(pl, tm, p, stream, true)));
     } else {
       GemmF32Params p = {};
       p.M = rows; p.N = ly.out; p.K = k_in;
@@ -478,27 +457,26 @@ int Net::enqueue_out(int rows, bool do_loss, bool do_bwd, float* yhat_dst, float
     p.g_wo = grad + ol.w_off; p.g_bo = grad + ol.b_off; p.g_bL = grad + hl.b_off;
   }
   const int grid = (rows + 31) / 32;
-  static const bool old_out = getenv("SB_OLD_OUT") != nullptr;
   if (tc()) {
     p.A = A[L - 1]; p.ldA = hl.ld_out;
     p.np = nparts; p.a_ps = A_ps[L - 1]; p.dz_ps = A_ps[L - 1];
     if (do_bwd) { p.dZ = dZ[L - 1]; p.ld_dZ = hl.ld_out; }
-    if (hl.out <= 1024 && !old_out) {
+    if (hl.out <= 1024) {
       // one-pass kernel: rows per block sized for ~2 blocks per SM, at least one row per warp
       int rpb = (rows + 2 * num_sms - 1) / (2 * num_sms);
       rpb = ((rpb + 7) / 8) * 8;
       if (rpb < 8) rpb = 8;
       const dim3 g((rows + rpb - 1) / rpb);
-      if (hl.out <= 256) SB_TRY(launch(out_layer_rows_kernel<1>, g, dim3(256), 0, stream, use_pdl, p, rpb));
-      else if (hl.out <= 512) SB_TRY(launch(out_layer_rows_kernel<2>, g, dim3(256), 0, stream, use_pdl, p, rpb));
-      else SB_TRY(launch(out_layer_rows_kernel<4>, g, dim3(256), 0, stream, use_pdl, p, rpb));
+      if (hl.out <= 256) SB_TRY(launch(out_layer_rows_kernel<1>, g, dim3(256), 0, stream, true, p, rpb));
+      else if (hl.out <= 512) SB_TRY(launch(out_layer_rows_kernel<2>, g, dim3(256), 0, stream, true, p, rpb));
+      else SB_TRY(launch(out_layer_rows_kernel<4>, g, dim3(256), 0, stream, true, p, rpb));
     } else {
-      SB_TRY(launch(out_layer_kernel<__nv_bfloat16>, dim3(grid), dim3(256), 0, stream, use_pdl, p));
+      SB_TRY(launch(out_layer_kernel<__nv_bfloat16>, dim3(grid), dim3(256), 0, stream, true, p));
     }
   } else {
     p.A = Af[L - 1]; p.ldA = hl.out;
     if (do_bwd) { p.dZ = dZf[L - 1]; p.ld_dZ = hl.out; }
-    SB_TRY(launch(out_layer_kernel<float>, dim3(grid), dim3(256), 0, stream, use_pdl, p));
+    SB_TRY(launch(out_layer_kernel<float>, dim3(grid), dim3(256), 0, stream, true, p));
   }
   SB_CUDA(cudaGetLastError());
   mark("out_layer");
@@ -508,48 +486,40 @@ int Net::enqueue_out(int rows, bool do_loss, bool do_bwd, float* yhat_dst, float
 int Net::enqueue_backward(int rows, float* grad) {
   // dW_l and dA_l both consume dZ_l and are independent of each other: the dW GEMMs go to the side stream and
   // overlap the dA chain (they are each well under one wave at cfg1 sizes).  Not while profiling (clean times).
-  const bool fork = concurrent_bwd && !profiling && side != nullptr && tc();
+  const bool fork = !profiling && side != nullptr && tc();
   // dW_1 (side stream) and dW_0 (main stream) run at the same time, one CTA per SM each.  If their natural grids do not
   // fit the machine together, dW_1's second wave only starts when dW_0's CTAs exit (measured: the side optimizer then
   // finishes 4 us after the main one, scripts/step_timeline.py).  Compare, in k-blocks per CTA, "natural grids, dW_1
   // finishing after dW_0" against "dW_1 on a third of the SMs, dW_0 on the rest" and take the shorter.
-  int dw_sms[2] = {gemm_sms, gemm_sms};
-  static const bool no_budget = getenv("SB_NO_DW_BUDGET") != nullptr;
+  int dw_sms[2] = {num_sms, num_sms};
   // dw1_serial_auto (single-GPU tail): when the natural grids of dW_0 and dW_1 do not fit the machine together, dW_1 runs IN
   // FRONT of dW_0 on the main stream instead of beside it - side by side the two persistent grids take turns on the SMs
   // (cfg2: 47.9 us for both; alone 13.9 + 29.0 us, profiles/ncu_r02_cfg2_launches.txt); small layers (cfg1) stay side by side
   bool dw1_front = dw1_first;
-  if (fork && dw0_on_main && L > 1 && !on_layer_grads && !no_budget && !dw1_last && !dw1_first) {
+  if (fork && dw0_on_main && L > 1 && !dw1_last && !dw1_first) {
     const int kx = round_up(rows, 64) * pairs_of(nparts);
-    const GemmPlan n0 = plan_gemm(layers[0].in, layers[0].out, kx, gemm_sms, true);
-    const GemmPlan n1 = plan_gemm(layers[1].in, layers[1].out, kx, gemm_sms, true);
-    if (n0.grid + n1.grid > gemm_sms && dw1_serial_auto && n0.cg == 2) {      // (pair tiles = a GEMM of several waves, plan_gemm)
+    const GemmPlan n0 = plan_gemm(layers[0].in, layers[0].out, kx, num_sms, true);
+    const GemmPlan n1 = plan_gemm(layers[1].in, layers[1].out, kx, num_sms, true);
+    if (n0.grid + n1.grid > num_sms && dw1_serial_auto && n0.cg == 2) {      // (pair tiles = a GEMM of several waves, plan_gemm)
       dw1_front = true;
-    } else if (n0.grid + n1.grid > gemm_sms) {
-      const GemmPlan b1 = plan_gemm(layers[1].in, layers[1].out, kx, gemm_sms / 3, true);
-      const GemmPlan b0 = plan_gemm(layers[0].in, layers[0].out, kx, gemm_sms - b1.grid, true);
+    } else if (n0.grid + n1.grid > num_sms) {
+      const GemmPlan b1 = plan_gemm(layers[1].in, layers[1].out, kx, num_sms / 3, true);
+      const GemmPlan b0 = plan_gemm(layers[0].in, layers[0].out, kx, num_sms - b1.grid, true);
       auto waves = [&](const GemmPlan& pl, int M, int N, int sms) {   // k-blocks one CTA works through
         const int tiles = ((M + 128 * pl.cg - 1) / (128 * pl.cg)) * ((N + pl.bn - 1) / pl.bn) * pl.split_k;
         const int slots = sms / pl.cg;
         return ((tiles + slots - 1) / slots) * pl.kb_per_split;
       };
-      const int t_nat = waves(n0, layers[0].in, layers[0].out, gemm_sms) + waves(n1, layers[1].in, layers[1].out, gemm_sms);
-      const int t0 = waves(b0, layers[0].in, layers[0].out, gemm_sms - b1.grid);
-      const int t1 = waves(b1, layers[1].in, layers[1].out, gemm_sms / 3);
-      if ((t0 > t1 ? t0 : t1) < t_nat) { dw_sms[1] = gemm_sms / 3; dw_sms[0] = gemm_sms - b1.grid; }
+      const int t_nat = waves(n0, layers[0].in, layers[0].out, num_sms) + waves(n1, layers[1].in, layers[1].out, num_sms);
+      const int t0 = waves(b0, layers[0].in, layers[0].out, num_sms - b1.grid);
+      const int t1 = waves(b1, layers[1].in, layers[1].out, num_sms / 3);
+      if ((t0 > t1 ? t0 : t1) < t_nat) { dw_sms[1] = num_sms / 3; dw_sms[0] = num_sms - b1.grid; }
     }
   }
   auto emit_dw_tc = [&](int l, bool force_main) -> int {
         Layer& ly = layers[l];
-        const long long wl_elems = static_cast<long long>(ly.in) * ly.out;
-        int n_chunks = 1;
-        if (fork && on_layer_grads && dw_chunk_bytes > 0 && (ly.out % 8) == 0 && wl_elems * 4 > 2 * dw_chunk_bytes) {
-          n_chunks = static_cast<int>((wl_elems * 4 + dw_chunk_bytes - 1) / dw_chunk_bytes);
-          if (n_chunks > 8) n_chunks = 8;
-        }
         const bool xchg_chunks = l == 0 && dw0_chunks >= 1 && on_dw0_chunk && (ly.out % 8 == 0 || dw0_chunks == 1) && !sparse_step;
-        if (xchg_chunks) n_chunks = dw0_chunks;
-        int chunk_rows = xchg_chunks ? dw0_chunk_rows() : round_up((ly.in + n_chunks - 1) / n_chunks, 128);
+        const int n_chunks = xchg_chunks ? dw0_chunks : 1;
         // dW_0 has nothing to overlap with (no dA_0): PDL-chained on the main stream right behind the last dA GEMM it
         // starts ~6 us earlier than as a cross-stream launch (measured, scripts/step_timeline.py)
         const bool on_main = !fork || (l == 0 && dw0_on_main && L > 1) || force_main;
@@ -561,13 +531,13 @@ int Net::enqueue_backward(int rows, float* grad) {
         const bool sp0 = (l == 0) && sparse_step;     // wide+deep: dW of the dense rows by GEMM, of the embedding rows by scatter-add
         const int in_rows = sp0 ? n_dense : ly.in;
         const int ld_k = sp0 ? ldD : ly.ld_in;
-        if (sp0) chunk_rows = round_up(in_rows, 128);
+        const int chunk_rows = xchg_chunks ? dw0_chunk_rows() : round_up(in_rows, 128);
         const __nv_bfloat16* ap = (l == 0) ? (res0 ? resident_Xb : Xb) : A[l - 1];
         const long long ap_ps = (l == 0) ? (res0 ? resident_ps : Xb_ps) : A_ps[l - 1];
         if (sp0) SB_TRY(enqueue_embed(rows, true, grad, on_main ? stream : side));
         for (int r0 = 0; r0 < in_rows; r0 += chunk_rows) {
           const int r1 = (r0 + chunk_rows < in_rows) ? r0 + chunk_rows : in_rows;
-          const GemmPlan pl = plan_gemm(r1 - r0, ly.out, round_up(rows, 64) * pairs_of(nparts), l < 2 ? dw_sms[l] : gemm_sms, true);
+          const GemmPlan pl = plan_gemm(r1 - r0, ly.out, round_up(rows, 64) * pairs_of(nparts), l < 2 ? dw_sms[l] : num_sms, true);
           TmapSet tm;
           // resident set: rows past the batch end are real rows of other batches; the B operand (dZ_l, extent = rows) is
           // zero-filled there, so they contribute nothing
@@ -580,16 +550,9 @@ int Net::enqueue_backward(int rows, float* grad) {
           p.accum = grad + ly.w_off + static_cast<long long>(r0) * ly.out; p.ld_acc = ly.out;
           p.acc_vec4 = (ly.out % 4 == 0 && ly.w_off % 4 == 0) ? 1 : 0;
           p.trace = next_trace("dW", l, r1 - r0, ly.out, rows, n_chunks > 1 ? r0 / chunk_rows : -1);
-          SB_TRY((launch_gemm_tc<EPI_DW, true, true>(pl, tm, p, on_main ? stream : side, use_pdl && on_main)));
+          SB_TRY((launch_gemm_tc<EPI_DW, true, true>(pl, tm, p, on_main ? stream : side, on_main)));
           mark("gemm_dw");
           if (xchg_chunks) SB_TRY(on_dw0_chunk(r0 / chunk_rows));
-          if (fork && on_layer_grads) {
-            const long long e0 = static_cast<long long>(r0) * ly.out, e1 = static_cast<long long>(r1) * ly.out;
-            SB_CUDA(cudaEventRecord(ev_dw[l], side));
-            SB_CUDA(cudaStreamWaitEvent(comm, ev_dw[l], 0));
-            SB_TRY(on_layer_grads(l, comm, 0, e0, e1));
-            if (l == 0) SB_TRY(on_layer_grads(l, comm, 1, e0, e1));  // no dA_0: W_0 is free to be updated
-          }
         }
         return SB_OK;
   };
@@ -597,8 +560,8 @@ int Net::enqueue_backward(int rows, float* grad) {
     Layer& ly = layers[l];
     if (tc()) {
       // dW_l[in,out] += sum_rows A_{l-1}[rows,in] (MN-major A) * dZ_l[rows,out] (MN-major B), split-K over rows.
-      // With a gradient exchange behind it, a big layer is cut into row chunks of W_l (each a contiguous slice of the
-      // flat gradient) so that the all-reduce of chunk c overlaps the GEMM of chunk c+1.
+      // With the peer exchange, dW_0 is cut into row chunks of W_0 (each a contiguous slice of the flat gradient) so that
+      // the exchange of chunk c overlaps the GEMM of chunk c+1.
       const bool dw1_moved = (dw1_last || dw1_front) && L > 1;
       if (dw1_front && l == 0 && L > 1) {         // in front of dW_0 on the main stream: dW_0's last exchange then runs on an idle GPU
         SB_TRY(emit_dw_tc(1, true));
@@ -609,7 +572,7 @@ int Net::enqueue_backward(int rows, float* grad) {
       if (l > 0) {
         // dZ_{l-1}[rows,in] = (dZ_l[rows,out] (K-major) x W_l[in,out] (K-major B: k = out contiguous)) .* act'(A_{l-1})
         Layer& pl = layers[l - 1];
-        const GemmPlan gp = plan_gemm(rows, ly.in, round_up(ly.out, 64) * pairs_of(nparts), gemm_sms, false);
+        const GemmPlan gp = plan_gemm(rows, ly.in, round_up(ly.out, 64) * pairs_of(nparts), num_sms, false);
         TmapSet tm;
         SB_TRY(make_tmaps_bf16(tm.a, dZ[l], A_ps[l], nparts, rows, ly.out, ly.ld_out, 128));
         SB_TRY(make_tmaps_bf16(tm.b, ly.Wn, Wn_ps[l], nparts, ly.in, ly.out, ly.ld_out, plan_box_rows_b(gp)));
@@ -625,14 +588,9 @@ int Net::enqueue_backward(int rows, float* grad) {
           SB_TRY(make_tmap_bf16(&tm.o, dZ[l - 1], rows, ly.in, pl.ld_out, 128));
           SB_TRY(make_tmap_bf16(&tm.x, A[l - 1], rows, ly.in, pl.ld_out, 128));
         }
-        SB_TRY((launch_gemm_tc<EPI_DA, false, false>(gp, tm, p, stream, use_pdl)));
+        SB_TRY((launch_gemm_tc<EPI_DA, false, false>(gp, tm, p, stream, true)));
         mark("gemm_da");
         if (l == 1 && fork && defer_join) SB_CUDA(cudaEventRecord(ev_da_done, stream));
-      }
-      if (fork && on_layer_grads && l > 0) {
-        SB_CUDA(cudaEventRecord(ev_da[l], stream));
-        SB_CUDA(cudaStreamWaitEvent(comm, ev_da[l], 0));
-        SB_TRY(on_layer_grads(l, comm, 1, 0, static_cast<long long>(ly.in) * ly.out));
       }
     } else {
       {
@@ -669,10 +627,6 @@ int Net::enqueue_backward(int rows, float* grad) {
   if (fork && !defer_join) {
     SB_CUDA(cudaEventRecord(ev_join, side));
     SB_CUDA(cudaStreamWaitEvent(stream, ev_join, 0));
-    if (on_layer_grads) {
-      SB_CUDA(cudaEventRecord(ev_comm, comm));
-      SB_CUDA(cudaStreamWaitEvent(stream, ev_comm, 0));
-    }
   }
   return SB_OK;
 }

@@ -26,27 +26,18 @@ struct Net {
   cudaStream_t side = nullptr;               // dW GEMMs run here, concurrently with the dA chain on `stream`
   std::vector<cudaEvent_t> ev_dz;            // ev_dz[l]: dZ_l is complete on `stream`
   cudaEvent_t ev_join = nullptr;
-  cudaStream_t comm = nullptr;               // per-layer gradient all-reduce + optimizer, pipelined behind the dW GEMMs
-  cudaStream_t comm2 = nullptr;              // second exchange stream (the chunk exchanges of hidden layer 0 alternate)
-  // Peer-exchange schedule (world > 1, set by the trainer around enqueue_backward / enqueue_hidden_forward):
+  cudaStream_t comm = nullptr;               // the peer exchanges of hidden layer 0's dW chunks alternate between
+  cudaStream_t comm2 = nullptr;              // these two streams
+  // Peer-exchange schedule (world > 1, set by the trainer around enqueue_backward):
   //   dW_0 runs on the main stream in `dw0_chunks` row chunks of W_0, on_dw0_chunk(c) is called behind each (its exchange
-  //   goes to a comm stream and overlaps the GEMMs that follow); dW_1 follows dW_0 on the main stream instead of running
-  //   beside it, so that the LAST chunk's exchange is covered too; before_layer1 is called in front of layer 1's forward
-  //   GEMM (the previous step's exchange of the other layers may still run beside the layer-0 forward GEMM);
-  //   zero_layer = the forward GEMM whose idle epilogue warps clear zero_buf (1: peers may still read the gradient
-  //   buffer while layer 0 runs).
+  //   goes to a comm stream and overlaps the GEMMs that follow); dW_1 runs on the main stream in front of dW_0 (dw1_first)
+  //   or behind it (dw1_last, so that the LAST chunk's exchange is covered too) instead of beside it.
   int dw0_chunks = 1;
   bool dw1_last = false;
   bool dw1_first = false;                    // dW_1 on the main stream IN FRONT of dW_0 (then after_dw1 is called behind it)
   std::function<int()> after_dw1;
   bool dw1_serial_auto = false;              // let enqueue_backward move dW_1 in front of dW_0 when their grids do not fit together
   std::function<int(int /*chunk*/)> on_dw0_chunk;
-  std::function<int()> before_layer1;
-  int zero_layer = 0;
-  // the previous step's exchange of slot 0 sits in front of this step on the main stream and has released its programmatic
-  // dependents at its start: the layer-0 forward GEMM skips its dependency wait (it runs BESIDE that exchange), and layer 1's
-  // forward is launched without the programmatic attribute, i.e. behind everything the stream has seen
-  bool beside_prev_xchg = false;
   int dw0_chunk_rows() const {
     const int c = dw0_chunks > 1 ? dw0_chunks : 1;
     return ((layers[0].in + c - 1) / c + 127) / 128 * 128;
@@ -59,20 +50,7 @@ struct Net {
   // optimizer per stream instead of joining first
   bool dw0_on_main = false, defer_join = false;
   cudaEvent_t ev_da_done = nullptr;          // the last dA GEMM (last reader of the bf16 weight shadows) is complete
-  std::vector<cudaEvent_t> ev_dw;            // ev_dw[l]: dW_l (and db_l) complete on `side`
-  cudaEvent_t ev_comm = nullptr;
-  // called (while enqueueing the backward pass) once the gradient segment of hidden layer l - and, for l = L-1, of
-  // the output layer that follows it in the flat layout - has been enqueued; work is expected on `comm`
-  // phase 0: dW_l enqueued (gradient segment complete) -> exchange; phase 1: dA_l enqueued too (W_l no longer read
-  // by this step) -> the optimizer may overwrite W_l and its bf16 shadow
-  // [e0, e1) = element range of W_l covered (chunked dW); e1 == in*out marks the chunk that completes the layer
-  std::function<int(int /*layer*/, cudaStream_t /*comm*/, int /*phase*/, long long /*e0*/, long long /*e1*/)> on_layer_grads;
-  int gemm_sms = 0;                          // SMs the persistent GEMMs may occupy (num_sms minus those left to NCCL)
-  long long dw_chunk_bytes = 0;              // > 0: split a layer's dW GEMM so each gradient chunk is about this big
-  std::vector<cudaEvent_t> ev_da;            // ev_da[l]: dA_l complete on `stream`
   std::vector<int> work_begin, work_end;     // optimizer work-table range of layer l (0..L)
-  bool concurrent_bwd = true;
-  bool use_pdl = true;                       // programmatic dependent launch along the main chain
   int F = 0, L = 0;             // features, hidden layers
   std::vector<Layer> layers;    // L hidden + 1 output (out = 1)
   long long n_params = 0;
@@ -178,8 +156,7 @@ struct Net {
   bool sparse_step = false;                  // set while a sparse step is being enqueued
   int set_sparse(int n_dense_, int n_onehot_, int n_cat_);
   int enqueue_embed(int rows, bool scatter, float* grad, cudaStream_t st);
-  bool fuse_out_layer = true;
-  int fuse_out_max = 256;                    // widest last hidden layer whose GEMM also runs the output layer (one n-tile)
+  static constexpr int fuse_out_max = 256;   // widest last hidden layer whose GEMM also runs the output layer (one n-tile)
   // bf16 HBM-resident training set (trainer): when `from_resident` is set while enqueueing, layer 0's GEMMs read their A
   // operand from it by TMA at row offset desc->row0 and no load_batch kernel runs (a sparse step: the set holds the dense
   // block, pitch ldD, and the embedding gather runs in front of the layer-0 forward GEMM)

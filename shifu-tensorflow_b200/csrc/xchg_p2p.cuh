@@ -72,10 +72,6 @@ struct XchgParams {
   unsigned int* host_err;                 // mapped pinned: [0] = 0 ok | 1 + 16 * slot + missing rank
   unsigned long long timeout_ns;          // 0 = wait forever
   int fence_gpu;                          // 1 (default): gpu-scope fence before the `updated` flag; SB_XCHG_FENCE_SYS=1 -> 0
-  int early_dependents;                   // 1: let the next kernel of the stream (PDL) become resident while this one still
-                                          // waits for its peers.  0 when the peers share this device (in-process replicas):
-                                          // the next step's persistent GEMM CTAs would take every SM's shared memory while
-                                          // they wait for this kernel, and the replica this kernel waits for could never run
   unsigned long long* trace;              // slots: 0 entry, 2 dependencies resolved, 3 every peer arrived (block 0), 4 last block's
                                           // runs done, 5 `updated` published, 6 every peer updated (block 0), 10 exit (gathered)
 };
@@ -136,8 +132,8 @@ __device__ __forceinline__ bool xchg_wait(const unsigned int* slots, int world, 
 
 // W = compile-time upper bound of `world`; a block iteration handles U consecutive runs with every load of the iteration in
 // flight before the first add.  <= 85 registers per thread: one block (21 k registers) fits beside ANY of the
-// persistent GEMM CTAs that may be resident while an exchange runs - the dW GEMMs of the same step (320 threads x 64) and
-// the next step's layer-0 forward (320 x <= 115) - so the exchange really overlaps them.
+// persistent GEMM CTAs that may be resident while an exchange runs - the dW GEMMs of the same step (320 threads x 64) -
+// so the exchange really overlaps them.
 // Measured on 2 x B200 through NVSwitch (scripts/p2p_probe.cu, profiles/p2p_probe_r02.txt): a flag takes 2.7 us one way, a
 // P2P load round trip ~5 us, bandwidth 750 GB/s only beyond ~16 MB in flight (4 MB: 14 us).  The chain arrive -> loads ->
 // stores + fence -> done therefore costs ~17 us however little data moves: the schedule (capi.cu) hides it behind GEMMs.
@@ -150,7 +146,6 @@ xchg_update_kernel(const XchgParams p) {
   if (threadIdx.x == 0) sh_fail = 0u;
   trace_begin(p.trace, true);
   pdl_wait();                 // the gradient of these slots is complete (stream order / programmatic dependency)
-  if (p.early_dependents) pdl_launch_dependents();
   trace_begin(p.trace, false);
   __syncthreads();
   const unsigned int epoch = p.desc->epoch;
@@ -485,7 +480,6 @@ xchg_ll_kernel(const LLParams lp) {
   if (threadIdx.x == 0) sh_fail = 0u;
   trace_begin(p.trace, true);
   pdl_wait();
-  if (p.early_dependents) pdl_launch_dependents();
   trace_begin(p.trace, false);
   __syncthreads();
   const unsigned int ep = p.desc->epoch;
